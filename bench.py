@@ -2,6 +2,7 @@
 """bench.py — the hot path (SA build + LUT + probe search + arm automaton + post-steps) on synthetic genomes.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..5] [--scale-n BP] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 One JSON line on rank 0. A "step" = one whole pass of the path over the workload genome:
@@ -145,6 +146,34 @@ def oracle_workload(config: int, scale_n: int):
 
 def searched_bp(prep) -> int:
     return int(sum(c[1] for c in prep.chunks))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _dump_rows(n: int, row_bytes: int, budget_bytes: int) -> np.ndarray:
+    """All n row numbers, or a fixed seeded sample of them (in order) when n rows would exceed the byte budget."""
+    if n * row_bytes <= budget_bytes:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=budget_bytes // row_bytes, replace=False))
+
+
+def dump_families(out_dir: str, fam) -> None:
+    """Write the families a caller of Context.search receives as <out_dir>/<field>.npy (float64; identity float32), so
+    that two builds can be compared output for output. Positions stay exact in float64 (< 2^53). Above 64 MB in all, a
+    fixed seeded sample of the family offsets (at most half the budget) and of the duplicons is written; fam_index.npy
+    and sd_index.npy hold the row numbers written."""
+    os.makedirs(out_dir, exist_ok=True)
+    sds = fam.sds
+    fields = ("left", "right", "left_length", "right_length", "identity", "reversed", "complemented")
+    fam_rows = _dump_rows(len(fam.fam_offsets), 16, DUMP_LIMIT_BYTES // 2)           # offset + row number
+    sd_rows = _dump_rows(len(sds), 8 * len(fields) + 4, DUMP_LIMIT_BYTES - 16 * len(fam_rows))   # identity is 4 B
+    out = {"fam_offsets": np.asarray(fam.fam_offsets, dtype=np.float64)[fam_rows], "fam_index": fam_rows.astype(np.float64),
+           "sd_index": sd_rows.astype(np.float64)}
+    for f in fields:
+        out[f] = sds[f][sd_rows].astype(np.float32 if f == "identity" else np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def golden(config: int):
@@ -387,6 +416,8 @@ def run_ours(args):
     ms, wall, fam = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
     stats = ctx.stats()
+    if args.dump_outputs and rank == 0:
+        dump_families(args.dump_outputs, fam)
     # ---- end to end through the C ABI with host buffers
     for _ in range(min(args.warmup, 3)):
         step_e2e()
@@ -532,7 +563,14 @@ def main():
     ap.add_argument("--check-sa", action="store_true", help="run the on-device sufcheck on every rank's index after the timed steps")
     ap.add_argument("--ref-sample-bp", type=int, default=0, help="--impl reference: genome length per step (0 = bounded default)")
     ap.add_argument("--no-ingest", action="store_true", help="skip the FASTA-ingest measurement (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the families of the last step as DIR/<field>.npy, to compare two "
+                         "builds of this project output for output (--impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computes")
     if args.impl == "reference":
         run_reference(args)
     else:
