@@ -72,6 +72,7 @@ class Stats(C.Structure):
         + [("ms_ingest", C.c_double), ("ingest_bytes", C.c_uint64), ("ingest_records", C.c_uint64)]
         + [(n, C.c_double) for n in ("ms_msd_scatter0", "ms_msd_hist", "ms_msd_local")]
         + [(n, C.c_uint64) for n in ("bytes_msd_scatter0", "bytes_msd_hist", "bytes_msd_local", "launches_msd_local", "msd_levels")]
+        + [("ms_locate", C.c_double)] + [(n, C.c_uint64) for n in ("locate_patterns", "locate_hits", "bytes_locate")]
     )
 
     def as_dict(self):
@@ -100,6 +101,8 @@ SYMBOLS = [
     "asgart_b200_ctx_build_index_trim", "asgart_b200_effective_trim", "asgart_b200_slice_families",
     "asgart_b200_run_files_sliced", "asgart_b200_run_files_sliced_ex", "asgart_b200_run_result_new", "asgart_b200_run_result_slice",
     "asgart_b200_run_result_to_json", "asgart_b200_run_result_error", "asgart_b200_run_result_free",
+    "asgart_b200_ctx_locate", "asgart_b200_hits_n_patterns", "asgart_b200_hits_first", "asgart_b200_hits_count",
+    "asgart_b200_hits_offsets", "asgart_b200_hits_positions", "asgart_b200_hits_free",
 ]
 
 _lib = None
@@ -145,6 +148,13 @@ def load() -> C.CDLL:
         "asgart_b200_ctx_download_lut": (i32, [vp, vp, vp]),
         "asgart_b200_ctx_search": (i32, [vp, vp, i64, PS, u32, C.POINTER(vp)]),
         "asgart_b200_ctx_probe_ranges": (i32, [vp, vp, PS, vp, vp, i64]),
+        "asgart_b200_ctx_locate": (i32, [vp, vp, vp, i64, i64, C.POINTER(vp)]),
+        "asgart_b200_hits_n_patterns": (i64, [vp]),
+        "asgart_b200_hits_first": (vp, [vp]),
+        "asgart_b200_hits_count": (vp, [vp]),
+        "asgart_b200_hits_offsets": (vp, [vp]),
+        "asgart_b200_hits_positions": (vp, [vp]),
+        "asgart_b200_hits_free": (None, [vp]),
         "asgart_b200_ctx_search_shard": (i32, [vp, vp, i64, PS, i32, i32, C.POINTER(vp)]),
         "asgart_b200_partial_size": (i64, [vp]),
         "asgart_b200_partial_serialize": (i32, [vp, vp, i64]),

@@ -138,6 +138,36 @@ def _take_result(L, rh) -> Families:
         L.asgart_b200_result_free(rh)
 
 
+@dataclass
+class Hits:
+    """Answer of Context.locate for a batch of patterns: sa_search64's (first, count) per pattern (count never capped) and
+    the reported positions, pattern i's being positions[offsets[i]:offsets[i+1]] = SA[first[i] : first[i] + min(count[i],
+    max_hits)], in suffix-array order."""
+    first: np.ndarray      # int64[n]
+    count: np.ndarray      # int64[n]
+    offsets: np.ndarray    # uint64[n + 1]
+    positions: np.ndarray  # int64[offsets[n]]
+
+    def positions_of(self, i: int) -> np.ndarray:
+        return self.positions[int(self.offsets[i]):int(self.offsets[i + 1])]
+
+
+def pattern_batch(patterns) -> Tuple[np.ndarray, np.ndarray]:
+    """(uint8 bytes, uint64 offsets[n + 1]) of a batch: a sequence of bytes / str, or such a pair already (for millions of
+    patterns without a Python loop)."""
+    if isinstance(patterns, tuple) and len(patterns) == 2 and isinstance(patterns[0], np.ndarray):
+        buf = np.ascontiguousarray(patterns[0], dtype=np.uint8).reshape(-1)
+        off = np.ascontiguousarray(patterns[1], dtype=np.uint64).reshape(-1)
+        if len(off) == 0 or int(off[-1]) != len(buf):
+            raise AsgartB200Error(_lib.EINVAL, "pattern offsets must have n + 1 entries, the last one the byte count")
+        return buf, off
+    items = [p.encode() if isinstance(p, str) else bytes(p) for p in patterns]
+    off = np.zeros(len(items) + 1, dtype=np.uint64)
+    if items:
+        np.cumsum([len(p) for p in items], out=off[1:])
+    return np.frombuffer(b"".join(items), dtype=np.uint8), off
+
+
 def device_count() -> int:
     return int(_lib.load().asgart_b200_device_count())
 
@@ -321,6 +351,33 @@ class Context:
         hi = np.empty(n_probes, dtype=np.int64)
         self._check(self.L.asgart_b200_ctx_probe_ranges(self.h, _ptr(ch), C.byref(st), _ptr(lo), _ptr(hi), n_probes))
         return lo, hi
+
+    def locate(self, patterns, max_hits: Optional[int] = None) -> Hits:
+        """Where each pattern occurs in the strand, from the resident index: libdivsufsort's sa_search64 for every pattern
+        of the batch (any bytes, compared as bytes) and up to ``max_hits`` positions each (None: all, 0: counts only).
+        ``patterns``: a sequence of bytes / str, or a (uint8 array, uint64 offsets[n + 1]) pair."""
+        buf, off = pattern_batch(patterns)
+        n = len(off) - 1
+        h = C.c_void_p()
+        self._check(self.L.asgart_b200_ctx_locate(self.h, _ptr(buf) if len(buf) else None, _ptr(off), n,
+                                                  -1 if max_hits is None else int(max_hits), C.byref(h)))
+        L = self.L
+        try:
+            def arr(ptr, ctype, k, dtype):
+                if k == 0:
+                    return np.zeros(0, dtype=dtype)
+                return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(ctype)), shape=(k,)).copy()
+            offsets = arr(L.asgart_b200_hits_offsets(h), C.c_uint64, n + 1, np.uint64)
+            return Hits(arr(L.asgart_b200_hits_first(h), C.c_int64, n, np.int64),
+                        arr(L.asgart_b200_hits_count(h), C.c_int64, n, np.int64), offsets,
+                        arr(L.asgart_b200_hits_positions(h), C.c_int64, int(offsets[-1]), np.int64))
+        finally:
+            L.asgart_b200_hits_free(h)
+
+    def sa_search(self, patterns) -> Tuple[np.ndarray, np.ndarray]:
+        """sa_search64 for every pattern of the batch: (first int64[n], count int64[n]); see locate."""
+        hits = self.locate(patterns, max_hits=0)
+        return hits.first, hits.count
 
     def search_shard(self, chunks, settings: RunSettings, shard: int, n_shards: int) -> bytes:
         """Stage A over this rank's probe range; returns the serialised partial (to be all-gathered)."""

@@ -2,6 +2,7 @@
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
 #include <thread>
@@ -18,6 +19,7 @@
 #include "host_internal.h"
 #include "sa_build.cuh"
 #include "levenshtein.cuh"
+#include "locate.cuh"
 #include "search.cuh"
 
 namespace ab200 {
@@ -87,6 +89,15 @@ struct asgart_b200_ctx {
     std::vector<IngestPiece> pieces;
     u8* stage[2] = {nullptr, nullptr};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
+    // ctx_locate: its kernels' device time, pinned staging of its copies
+    FamilyTimer t_locate;
+    u8* loc_stage = nullptr;
+};
+
+struct asgart_b200_hits {
+    std::vector<int64_t> first, count;
+    std::vector<uint64_t> offsets;
+    std::vector<int64_t> positions;
 };
 
 namespace ab200 { namespace detail {
@@ -911,8 +922,141 @@ void fold_family_timers(asgart_b200_ctx* ctx) {
     S.bytes_sa_scatter_main = ctx->t_scatter_main.bytes;
     S.ms_sa_scatter = ctx->t_scatter.total_ms + S.ms_sa_scatter_main; S.launches_sa_scatter = ctx->t_scatter.launches + S.launches_sa_scatter_main;
     S.bytes_sa_scatter = ctx->t_scatter.bytes + S.bytes_sa_scatter_main;
+    ctx->t_locate.drain();
+    S.ms_locate = ctx->t_locate.total_ms;
     S.launches_total = ctx->launches.total;
     S.sa_index_bits = u64(ctx->idx_bits);
+}
+
+
+// ---- ctx_locate (locate.cuh) -----------------------------------------------------------------------------------
+constexpr u64 kLocSliceBytes = u64(1) << 28;      // pattern bytes on the device at a time
+constexpr u64 kLocSlicePatterns = u64(1) << 24;   // patterns on the device at a time (list entries are u32)
+constexpr u64 kLocWindow = u64(1) << 26;          // positions per copy launch (512 MB of int64)
+constexpr size_t kLocStage = size_t(1) << 25;     // pinned staging buffer of the host copies
+
+// host <-> device through the context's pinned staging buffer, on its stream
+void loc_copy(asgart_b200_ctx* ctx, void* dst, const void* src, size_t bytes, bool to_device) {
+    if (!bytes) return;
+    if (!ctx->loc_stage) CUDA_CHECK(cudaHostAlloc(reinterpret_cast<void**>(&ctx->loc_stage), kLocStage, cudaHostAllocDefault));
+    for (size_t o = 0; o < bytes; o += kLocStage) {
+        const size_t m = std::min(kLocStage, bytes - o);
+        if (to_device) {
+            memcpy(ctx->loc_stage, static_cast<const u8*>(src) + o, m);
+            CUDA_CHECK(cudaMemcpyAsync(static_cast<u8*>(dst) + o, ctx->loc_stage, m, cudaMemcpyHostToDevice, ctx->stream));
+            CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+        } else {
+            CUDA_CHECK(cudaMemcpyAsync(ctx->loc_stage, static_cast<const u8*>(src) + o, m, cudaMemcpyDeviceToHost, ctx->stream));
+            CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+            memcpy(static_cast<u8*>(dst) + o, ctx->loc_stage, m);
+        }
+    }
+    (to_device ? ctx->st.h2d_bytes : ctx->st.d2h_bytes) += bytes;
+}
+
+// returns false when the positions do not fit in host memory
+template <typename IdxT>
+bool locate_t(asgart_b200_ctx* ctx, const u8* patterns, const u64* offsets, u64 n, i64 max_hits, asgart_b200_hits& H) {
+    auto& ix = IxOf<IdxT>::get(ctx);
+    cudaStream_t s = ctx->stream;
+    const bool literal = ctx->sa_len != ctx->n1;   // --trim: the literal search (SURVEY Q9)
+    const u64 cap = max_hits < 0 ? ~u64(0) : u64(max_hits);
+    H.first.assign(n, 0);
+    H.count.assign(n, 0);
+    H.offsets.assign(n + 1, 0);
+    DevBuf<unsigned long long> d_alg(1, s);
+    d_alg.zero();
+    u64 hits = 0;
+    for (u64 p0 = 0; p0 < n;) {
+        u64 p1 = p0 + 1;   // a slice: bounded bytes and patterns (a single longer pattern makes a slice of its own)
+        while (p1 < n && p1 - p0 < kLocSlicePatterns && offsets[p1 + 1] - offsets[p0] <= kLocSliceBytes) ++p1;
+        const u64 np = p1 - p0, base = offsets[p0], nb = offsets[p1] - base, nw = ceil_div(nb, 16) + 4;
+        std::vector<u64> off(np + 1);
+        for (u64 i = 0; i <= np; ++i) off[i] = offsets[p0 + i] - base;
+        std::vector<u32> list_short, list_long;   // keeps the long patterns out of the warps of the short ones
+        if (!literal)
+            for (u64 i = 0; i < np; ++i) (off[i + 1] - off[i] <= 32 ? list_short : list_long).push_back(u32(i));
+        DevBuf<u8> d_pat(nb, s);
+        DevBuf<u64> d_off(np + 1, s), d_pp(nw, s), d_cut(np, s);
+        DevBuf<i64> d_first(np, s), d_count(np, s);
+        DevBuf<u32> d_short(list_short.size(), s), d_long(list_long.size(), s);
+        loc_copy(ctx, d_pat.p, patterns + base, nb, true);
+        loc_copy(ctx, d_off.p, off.data(), (np + 1) * 8, true);
+        loc_copy(ctx, d_short.p, list_short.data(), list_short.size() * 4, true);
+        loc_copy(ctx, d_long.p, list_long.data(), list_long.size() * 4, true);
+        CUDA_CHECK(cudaMemsetAsync(d_cut.p, 0xFF, np * 8, s));
+        locate_pack_kernel<<<unsigned(ceil_div(nw, 256)), 256, 0, s>>>(d_pat.p, nb, d_off.p, np, d_pp.p, nw,
+                                                                      reinterpret_cast<unsigned long long*>(d_cut.p));
+        KERNEL_CHECK();
+        count_launch();
+        LocateParams<IdxT> P{};
+        P.PT = ctx->d_pt.p; P.n1 = ctx->n1; P.SA = ix.sa.p; P.sa_len = ctx->sa_len;
+        P.lut_lo = ix.lut_lo.p; P.lut_hi = ix.lut_hi.p; P.deep = ix.deep.p; P.deep_depth = ix.deep.p ? ix.deep_depth : 0;
+        P.pat = d_pat.p; P.PP = d_pp.p; P.off = d_off.p; P.cut = d_cut.p;
+        P.first = d_first.p; P.count = d_count.p; P.alg_bytes = d_alg.p;
+        ctx->t_locate.begin();
+        u64 launches = 0;
+        if (literal) {
+            P.list = nullptr; P.n_list = np;
+            locate_literal_kernel<IdxT><<<unsigned(ceil_div(np, 256)), 256, 0, s>>>(P);
+            KERNEL_CHECK();
+            ++launches;
+        } else {
+            if (!list_short.empty()) {
+                P.list = d_short.p; P.n_list = list_short.size();
+                locate_short_kernel<IdxT><<<unsigned(ceil_div(P.n_list, 256)), 256, 0, s>>>(P);
+                KERNEL_CHECK();
+                ++launches;
+            }
+            if (!list_long.empty()) {
+                P.list = d_long.p; P.n_list = list_long.size();
+                locate_long_kernel<IdxT><<<unsigned(ceil_div(P.n_list * 32, 256)), 256, 0, s>>>(P);
+                KERNEL_CHECK();
+                ++launches;
+            }
+        }
+        ctx->t_locate.end(launches, 0);
+        count_launch(launches);
+        loc_copy(ctx, H.first.data() + p0, d_first.p, np * 8, false);
+        loc_copy(ctx, H.count.data() + p0, d_count.p, np * 8, false);
+        u64 hs = 0;
+        for (u64 i = 0; i < np; ++i) {
+            hs += std::min(u64(H.count[p0 + i]), cap);
+            H.offsets[p0 + i + 1] = hits + hs;
+        }
+        if (hs) {
+            try {
+                H.positions.resize(hits + hs);
+            } catch (const std::exception&) {
+                return false;
+            }
+            DevBuf<u64> d_moff(np, s);
+            const i64* cp = d_count.p;
+            u64* mp = d_moff.p;
+            device_scan<u64, SumOp>([cp, cap] __device__(u64 i) { const u64 c = u64(cp[i]); return c < cap ? c : cap; },
+                                    [mp] __device__(u64 i, u64 exc, u64) { mp[i] = exc; }, np, (u64*)nullptr, s);
+            DevBuf<i64> d_out(std::min(hs, kLocWindow), s);
+            for (u64 w0 = 0; w0 < hs; w0 += kLocWindow) {
+                const u64 w1 = std::min(hs, w0 + kLocWindow);
+                ctx->t_locate.begin();
+                locate_copy_kernel<IdxT><<<unsigned(ceil_div(np * 32, 256)), 256, 0, s>>>(ix.sa.p, d_first.p, d_count.p, d_moff.p, np,
+                                                                                         cap, w0, w1, d_out.p);
+                KERNEL_CHECK();
+                ctx->t_locate.end(1, 0);
+                count_launch();
+                loc_copy(ctx, H.positions.data() + hits + w0, d_out.p, (w1 - w0) * 8, false);
+            }
+        }
+        hits += hs;
+        p0 = p1;
+    }
+    unsigned long long alg = 0;
+    CUDA_CHECK(cudaMemcpyAsync(&alg, d_alg.p, sizeof alg, cudaMemcpyDeviceToHost, s));
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    ctx->st.locate_patterns += n;
+    ctx->st.locate_hits += hits;
+    ctx->st.bytes_locate += u64(alg) + 8 * hits;
+    return true;
 }
 
 } }  // namespace ab200::detail
@@ -948,6 +1092,7 @@ int32_t asgart_b200_ctx_create(int32_t device, asgart_b200_ctx** out) {
         ctx->t_sort.init(ctx->stream); ctx->t_gather.init(ctx->stream); ctx->t_rank.init(ctx->stream);
         ctx->t_probe.init(ctx->stream); ctx->t_emit.init(ctx->stream); ctx->t_scatter.init(ctx->stream); ctx->t_scatter_main.init(ctx->stream);
         ctx->t_msd0.init(ctx->stream); ctx->t_msd_hist.init(ctx->stream); ctx->t_msd_local.init(ctx->stream);
+        ctx->t_locate.init(ctx->stream);
         CUDA_CHECK(cudaEventCreate(&ctx->ev_a)); CUDA_CHECK(cudaEventCreate(&ctx->ev_b));
     } catch (const CudaError& e) {
         int code = e.code;
@@ -967,7 +1112,8 @@ void asgart_b200_ctx_destroy(asgart_b200_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     ctx->t_sort.destroy(); ctx->t_gather.destroy(); ctx->t_rank.destroy(); ctx->t_probe.destroy(); ctx->t_emit.destroy(); ctx->t_scatter.destroy(); ctx->t_scatter_main.destroy();
-    ctx->t_msd0.destroy(); ctx->t_msd_hist.destroy(); ctx->t_msd_local.destroy();
+    ctx->t_msd0.destroy(); ctx->t_msd_hist.destroy(); ctx->t_msd_local.destroy(); ctx->t_locate.destroy();
+    if (ctx->loc_stage) cudaFreeHost(ctx->loc_stage);
     if (ctx->ev_a) cudaEventDestroy(ctx->ev_a);
     if (ctx->ev_b) cudaEventDestroy(ctx->ev_b);
     if (ctx->group_owned && ctx->group) { delete ctx->group; }
@@ -1669,6 +1815,34 @@ const uint64_t* asgart_b200_result_family_offsets(const asgart_b200_result* r) {
 const asgart_b200_protosd* asgart_b200_result_sds(const asgart_b200_result* r) { return r ? r->sds.data() : nullptr; }
 void asgart_b200_result_free(asgart_b200_result* r) { delete r; }
 
+// ---- exact-match queries (locate.cuh) --------------------------------------------------------------------------
+int32_t asgart_b200_ctx_locate(asgart_b200_ctx* ctx, const uint8_t* patterns, const uint64_t* offsets, int64_t n_patterns,
+                               int64_t max_hits, asgart_b200_hits** out) {
+    if (asgart_b200_device_count() <= 0) return ASGART_B200_ENODEVICE;
+    return guarded(ctx, [&]() -> int32_t {
+        if (!out) return fail(ctx, ASGART_B200_EINVAL, "null out");
+        *out = nullptr;
+        if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "locate before build_index");
+        if (n_patterns < 0 || (n_patterns > 0 && !offsets)) return fail(ctx, ASGART_B200_EINVAL, "locate: bad pattern count or null offsets");
+        const u64 n = u64(n_patterns);
+        for (u64 i = 0; i < n; ++i)
+            if (offsets[i + 1] < offsets[i]) return fail(ctx, ASGART_B200_EINVAL, "locate: offsets are not non-decreasing");
+        if (n > 0 && offsets[n] > offsets[0] && !patterns) return fail(ctx, ASGART_B200_EINVAL, "locate: null patterns");
+        std::unique_ptr<asgart_b200_hits> H(new asgart_b200_hits());
+        const bool ok = ctx->idx_bits == 32 ? locate_t<u32>(ctx, patterns, offsets, n, max_hits, *H)
+                                            : locate_t<u64>(ctx, patterns, offsets, n, max_hits, *H);
+        if (!ok) return fail(ctx, ASGART_B200_ENOMEM, "locate: the reported positions do not fit in host memory (lower max_hits)");
+        *out = H.release();
+        return ASGART_B200_OK;
+    });
+}
+int64_t asgart_b200_hits_n_patterns(const asgart_b200_hits* h) { return h ? int64_t(h->first.size()) : 0; }
+const int64_t* asgart_b200_hits_first(const asgart_b200_hits* h) { return h ? h->first.data() : nullptr; }
+const int64_t* asgart_b200_hits_count(const asgart_b200_hits* h) { return h ? h->count.data() : nullptr; }
+const uint64_t* asgart_b200_hits_offsets(const asgart_b200_hits* h) { return h ? h->offsets.data() : nullptr; }
+const int64_t* asgart_b200_hits_positions(const asgart_b200_hits* h) { return h ? h->positions.data() : nullptr; }
+void asgart_b200_hits_free(asgart_b200_hits* h) { delete h; }
+
 int32_t asgart_b200_ctx_stats(const asgart_b200_ctx* ctx, asgart_b200_stats* out) {
     if (!ctx || !out) return ASGART_B200_EINVAL;
     asgart_b200_ctx* c = const_cast<asgart_b200_ctx*>(ctx);
@@ -1688,7 +1862,7 @@ void asgart_b200_ctx_reset_stats(asgart_b200_ctx* ctx) {
     try {
         cudaSetDevice(ctx->device);
         ctx->t_sort.reset(); ctx->t_gather.reset(); ctx->t_rank.reset(); ctx->t_probe.reset(); ctx->t_emit.reset(); ctx->t_scatter.reset(); ctx->t_scatter_main.reset();
-        ctx->t_msd0.reset(); ctx->t_msd_hist.reset(); ctx->t_msd_local.reset();
+        ctx->t_msd0.reset(); ctx->t_msd_hist.reset(); ctx->t_msd_local.reset(); ctx->t_locate.reset();
     } catch (...) {}
     ctx->launches.total = 0;
     ctx->st = asgart_b200_stats{};

@@ -172,6 +172,27 @@ ASGART_B200_API int32_t asgart_b200_ctx_probe_ranges(asgart_b200_ctx *ctx, const
                                                      const asgart_b200_settings *settings, int64_t *lo, int64_t *hi,
                                                      int64_t n_probes);
 
+/* ---- exact-match queries against the resident index ------------------------------------------------------------
+ * sa_search64 (libdivsufsort/lib/utils.c:282-349; bound by the reference at src/divsufsort.rs) for a batch of patterns
+ * against the context's index; pattern i = patterns[offsets[i] .. offsets[i+1]) (offsets: n_patterns + 1 entries,
+ * non-decreasing). Patterns are any bytes, compared as bytes (_compare, utils.c:244-255; a suffix that ends inside the
+ * pattern is smaller). Per pattern: count = number of suffixes that start with it, SA[first .. first + count) = those
+ * suffixes; count == 0: first = the reference's insertion point; the empty pattern: first 0, count = entries of the index.
+ * On an index built with --trim the answer is the one the reference's own bisection lands on (that array is not sorted
+ * for the whole strand it is compared with, SURVEY Q9).
+ * max_hits: positions reported per pattern (< 0 all, 0 counts only): SA[first .. first + min(count, max_hits)), in SA
+ * order; count itself is never capped. After build_index / build_index_trim / upload_sa. Device memory beyond the index
+ * stays bounded (patterns are taken in slices); ASGART_B200_ENOMEM when the positions do not fit in host memory. */
+typedef struct asgart_b200_hits asgart_b200_hits;
+ASGART_B200_API int32_t asgart_b200_ctx_locate(asgart_b200_ctx *ctx, const uint8_t *patterns, const uint64_t *offsets,
+                                               int64_t n_patterns, int64_t max_hits, asgart_b200_hits **out);
+ASGART_B200_API int64_t asgart_b200_hits_n_patterns(const asgart_b200_hits *h);
+ASGART_B200_API const int64_t *asgart_b200_hits_first(const asgart_b200_hits *h);      /* n_patterns */
+ASGART_B200_API const int64_t *asgart_b200_hits_count(const asgart_b200_hits *h);      /* n_patterns, uncapped */
+ASGART_B200_API const uint64_t *asgart_b200_hits_offsets(const asgart_b200_hits *h);   /* n_patterns + 1 */
+ASGART_B200_API const int64_t *asgart_b200_hits_positions(const asgart_b200_hits *h);  /* offsets[n_patterns] */
+ASGART_B200_API void asgart_b200_hits_free(asgart_b200_hits *h);
+
 /* Multi-GPU (one process per GPU; strand + index replicated; probes partitioned by position):
  *   every rank: ctx_search_shard(rank, world) -> partial; exchange the serialised partials (NCCL all-gather);
  *   any rank:   ctx_finish(partials[world]) -> families (identical on every rank and for every world size). */
@@ -239,6 +260,10 @@ typedef struct asgart_b200_stats {
      * builds the keys from the text, the per-level histograms, the in-shared-memory finishing sort, levels used */
     double ms_msd_scatter0, ms_msd_hist, ms_msd_local;
     uint64_t bytes_msd_scatter0, bytes_msd_hist, bytes_msd_local, launches_msd_local, msd_levels;
+    /* asgart_b200_ctx_locate: accumulated device ms of its search and copy kernels, patterns, reported positions and
+     * algorithmic bytes (24 B per bisection step, 16 B per further 32 symbols compared, 8 B per reported position) */
+    double ms_locate;
+    uint64_t locate_patterns, locate_hits, bytes_locate;
 } asgart_b200_stats;
 ASGART_B200_API int32_t asgart_b200_ctx_stats(const asgart_b200_ctx *ctx, asgart_b200_stats *out);
 ASGART_B200_API void asgart_b200_ctx_reset_stats(asgart_b200_ctx *ctx);
