@@ -90,7 +90,7 @@ SYMBOLS = [
     "asgart_b200_ctx_search_shard_dev", "asgart_b200_ctx_finish_dev",
     "asgart_b200_result_n_families", "asgart_b200_result_n_sds", "asgart_b200_result_family_offsets",
     "asgart_b200_result_sds", "asgart_b200_result_free", "asgart_b200_ctx_post_steps", "asgart_b200_ctx_stats",
-    "asgart_b200_ctx_reset_stats", "asgart_b200_ctx_timer_start", "asgart_b200_ctx_timer_stop", "asgart_b200_prepare_files", "asgart_b200_prepare_memory",
+    "asgart_b200_ctx_reset_stats", "asgart_b200_ctx_probe_keys", "asgart_b200_ctx_timer_start", "asgart_b200_ctx_timer_stop", "asgart_b200_prepare_files", "asgart_b200_prepare_memory",
     "asgart_b200_prepared_strand", "asgart_b200_prepared_chunks", "asgart_b200_prepared_n_fragments",
     "asgart_b200_prepared_fragment", "asgart_b200_prepared_free", "asgart_b200_to_json", "asgart_b200_free_string",
     "asgart_b200_out_filename", "asgart_b200_run_files", "asgart_b200_synth_length", "asgart_b200_synth_fill",
@@ -170,6 +170,7 @@ def load() -> C.CDLL:
         "asgart_b200_ctx_post_steps": (i32, [vp, vp, i64, vp, u32, C.POINTER(vp)]),
         "asgart_b200_ctx_stats": (i32, [vp, C.POINTER(Stats)]),
         "asgart_b200_ctx_reset_stats": (None, [vp]),
+        "asgart_b200_ctx_probe_keys": (C.c_uint64, [vp]),
         "asgart_b200_ctx_timer_start": (i32, [vp]),
         "asgart_b200_ctx_timer_stop": (i32, [vp, C.POINTER(C.c_double)]),
         "asgart_b200_prepare_files": (vp, [C.c_char_p, i32, C.POINTER(C.c_char_p)]),

@@ -436,7 +436,8 @@ class Context:
     def stats(self) -> dict:
         s = _lib.Stats()
         self._check(self.L.asgart_b200_ctx_stats(self.h, C.byref(s)))
-        return s.as_dict()
+        # n_probe_keys: probes answered from the sorted keys kept with the index (asgart_b200_ctx_probe_keys)
+        return s.as_dict() | {"n_probe_keys": int(self.L.asgart_b200_ctx_probe_keys(self.h))}
 
     def reset_stats(self):
         self.L.asgart_b200_ctx_reset_stats(self.h)

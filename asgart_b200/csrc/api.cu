@@ -27,8 +27,11 @@ thread_local LaunchCounter* g_launch_counter = nullptr;
 thread_local HostStalls g_host_stalls;   // per thread: the members of build_index_group count their own stalls
 thread_local DevicePool* g_device_pool = nullptr;
 
-struct Index32 { DevBuf<u32> sa, lut_lo, lut_hi, deep; int deep_depth = 0; };
-struct Index64 { DevBuf<u64> sa, lut_lo, lut_hi, deep; int deep_depth = 0; };
+// keys: the build's sorted initial keys (keys[i] = first key_p0 symbols of suffix SA[i], key_b bits each, first symbol on
+// top), kept for the probe search when build_index ran on one device with lazy ranks; key_map = strand code (CODE_*) ->
+// key code, one nibble each (0xF: the symbol does not occur in the strand)
+struct Index32 { DevBuf<u32> sa, lut_lo, lut_hi, deep; int deep_depth = 0; DevBuf<u64> keys; int key_b = 0, key_p0 = 0; u64 key_map = 0; };
+struct Index64 { DevBuf<u64> sa, lut_lo, lut_hi, deep; int deep_depth = 0; DevBuf<u64> keys; int key_b = 0, key_p0 = 0; u64 key_map = 0; };
 
 struct ChunkPlan {
     std::vector<ChunkDev> host;
@@ -91,6 +94,7 @@ struct asgart_b200_ctx {
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
     // ctx_locate: its kernels' device time, pinned staging of its copies
     FamilyTimer t_locate;
+    u64 n_probe_keys = 0;   // asgart_b200_ctx_probe_keys
     u8* loc_stage = nullptr;
 };
 
@@ -206,6 +210,10 @@ template <typename IdxT> struct IxOf;
 template <> struct IxOf<u32> { static Index32& get(asgart_b200_ctx* c) { return c->ix32; } };
 template <> struct IxOf<u64> { static Index64& get(asgart_b200_ctx* c) { return c->ix64; } };
 
+// the sorted keys describe the strand and the index they were built with: a new strand, a new index or another index
+// width makes them stale
+void drop_sorted_keys(asgart_b200_ctx* ctx) { ctx->ix32.keys.release(); ctx->ix64.keys.release(); }
+
 int pick_bits(const asgart_b200_ctx* ctx) {
     if (ctx->want_bits == 32 || ctx->want_bits == 64) return ctx->want_bits;
     return (ctx->n1 < 0xFFFFFFFEull) ? 32 : 64;
@@ -221,6 +229,7 @@ void build_lut(asgart_b200_ctx* ctx) {
     ix.lut_hi.zero();
     ix.deep.release();
     ix.deep_depth = 0;
+    ix.keys.release();
     lut_build_kernel<IdxT><<<unsigned(ceil_div(ctx->n1, 256)), 256, 0, ctx->stream>>>(ctx->d_pt.p, ix.sa.p, ctx->n1, ix.lut_lo.p,
                                                                                       ix.lut_hi.p);
     KERNEL_CHECK();
@@ -241,6 +250,9 @@ struct LutHook : SaKeyHook {
         t.deep = ix.deep.p; t.depth = ix.deep_depth; t.lut_lo = ix.lut_lo.p; t.lut_hi = ix.lut_hi.p; t.m4 = m4; t.m5 = m5;
         return ix.deep.p != nullptr;
     }
+    void adopt_sorted_keys(DevBuf<u64>& keys) override {
+        if (done) IxOf<IdxT>::get(ctx).keys = std::move(keys);
+    }
     void on_sorted_keys(const u64* d_keys, u64 n_local, u64 base, u64 n, int b, int p0, const uint16_t* h_code, cudaStream_t stream,
                         SaGroup* grp) override {
         if (p0 < 8 || n != ctx->n1) return;
@@ -254,6 +266,11 @@ struct LutHook : SaKeyHook {
         for (int d = 0; d < 5; ++d) if (h_code[u8(s5[d])] && h_code[u8(s5[d])] < 16) map.d5[h_code[u8(s5[d])]] = u8(d);
         for (int d = 0; d < 4; ++d) if (h_code[u8(s4[d])] && h_code[u8(s4[d])] < 16) map.d4[h_code[u8(s4[d])]] = u8(d);
         m4 = map.nibbles(map.d4); m5 = map.nibbles(map.d5);
+        ix.key_b = b; ix.key_p0 = p0; ix.key_map = ~u64(0);
+        for (const char* c = "$ACGNT"; *c; ++c) {
+            const u32 code = code_of_byte(u8(*c)), dense = h_code[u8(*c)];
+            if (dense && dense < 16) ix.key_map = (ix.key_map & ~(u64(15) << (4 * code))) | (u64(dense) << (4 * code));
+        }
         // depth: buckets of a few suffixes (4^depth <= n), at most 15 symbols (4 GiB of u32 starts: buckets of ~3 suffixes
         // for a 3.1 Gbp strand, which one round of parallel loads compares, instead of a bisection), inside the initial key
         static const int depth_cap = std::min(15, getenv("ASGART_B200_DEEP_MAX") ? atoi(getenv("ASGART_B200_DEEP_MAX")) : 15);
@@ -365,6 +382,7 @@ template <typename IdxT>
 void build_index_t(asgart_b200_ctx* ctx) {
     NvtxRange nv("build_index");
     auto& ix = IxOf<IdxT>::get(ctx);
+    ix.keys.release();   // before the sort allocates its key buffers: they take this block again
     EventTimer tsa(ctx->stream), tlut(ctx->stream);
     tsa.start();
     ix.sa.alloc(ctx->n1, ctx->stream);
@@ -410,6 +428,7 @@ void build_index_t(asgart_b200_ctx* ctx) {
 template <typename IdxT>
 void build_index_trim_t(asgart_b200_ctx* ctx, u64 a, u64 b) {
     auto& ix = IxOf<IdxT>::get(ctx);
+    ix.keys.release();
     cudaStream_t s = ctx->stream;
     EventTimer tsa(s), tlut(s);
     tsa.start();
@@ -594,9 +613,10 @@ void ensure_needle(asgart_b200_ctx* ctx, int mode) {
 
 // ---------------------------------------------------------------------------------------------- stage A
 // probe_search_kernel over [p_begin, p_end) and, when the deep table is usable (k >= its depth), probe_deferred_kernel over
-// the probes it left to the literal search. Reads the counters back (one sync).
+// the probes it left to the literal search. Reads the counters back (one sync). mode: the needle image (PackMode).
+// Returns the number of probes answered from the sorted keys.
 template <typename IdxT>
-void run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, unsigned long long* h_ctr) {
+u64 run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, int mode, unsigned long long* h_ctr) {
     auto& ix = IxOf<IdxT>::get(ctx);
     cudaStream_t s = ctx->stream;
     const u64 np = P.p_end - P.p_begin;
@@ -611,15 +631,32 @@ void run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, unsigned long
         deferred.alloc(np, s);
         P.deep = ix.deep.p; P.deep_depth = ix.deep_depth; P.q6_bits = q6.p; P.deferred = deferred.p;
     }
-    // shape (LINEAR = 8 suffixes compared at once, 2 blocks per SM = 128 registers) picked on B200 at C4 size: more
-    // blocks per SM or a shorter LINEAR are slower, the kernel is bound by random DRAM sectors (profiles/r1_experiments.log)
-    probe_search_kernel<IdxT, 8, 2><<<unsigned(ceil_div(np, 256)), 256, 0, s>>>(P);
+    // The deep buckets are compared in the sorted keys when the build left them, and when every symbol of the needle
+    // image has a key code: the codes are those of the bytes that occur in the strand, so a strand with A but no T,
+    // searched with its complement, compares on the text.
+    bool keys = deep && ix.keys.p;
+    const auto has_code = [&](u32 c) { return ((ix.key_map >> (4 * c)) & 15u) != 15u; };
+    for (u32 c : {CODE_A, CODE_C, CODE_G, CODE_N, CODE_T})
+        if (has_code(c) && !has_code((mode & PACK_COMPLEMENT) ? complement_code(c) : c)) keys = false;
+    if (keys) { P.keys = ix.keys.p; P.key_b = ix.key_b; P.key_p0 = ix.key_p0; P.key_map = ix.key_map; }
+    // shape of the text comparison (LINEAR = 8 suffixes compared at once, 2 blocks per SM = 128 registers) picked on B200
+    // at C4 size: more blocks per SM or a shorter LINEAR are slower, the kernel is bound by random DRAM sectors
+    // (profiles/r1_experiments.log). The keys comparison needs 71 (u32) / 75 (u64) registers at that shape, no spills;
+    // tried on one B200 (1000 W) at C4 size, while the counters still took one atomic per warp: LINEAR 4, 8, 16 with 2, 3,
+    // 4 blocks per SM all within 1 ms of each other (LINEAR 4 with 4 blocks: 44.0 ms, this shape: 44.2 ms), so it keeps
+    // the text comparison's shape (22.2 ms with the per-block counters; the other shapes were not timed again).
+    if (keys) probe_search_kernel<IdxT, 8, 2, true><<<unsigned(ceil_div(np, 256)), 256, 0, s>>>(P);
+    else probe_search_kernel<IdxT, 8, 2, false><<<unsigned(ceil_div(np, 256)), 256, 0, s>>>(P);
     KERNEL_CHECK();
     count_launch();
+    u64 n_keys = 0;
     if (deep) {
-        unsigned long long n_def = 0;
-        CUDA_CHECK(cudaMemcpyAsync(&n_def, P.counters + CTR_DEFERRED, sizeof n_def, cudaMemcpyDeviceToHost, s));
+        // with the keys, every probe probe_search_kernel searched itself was answered from them (it defers all others)
+        unsigned long long first[CTR_DEFERRED + 1];
+        CUDA_CHECK(cudaMemcpyAsync(first, P.counters, sizeof first, cudaMemcpyDeviceToHost, s));
         CUDA_CHECK(cudaStreamSynchronize(s));
+        const u64 n_def = first[CTR_DEFERRED];
+        if (keys) n_keys = first[CTR_SEARCHED];
         if (n_def) {
             probe_deferred_kernel<IdxT><<<unsigned(ceil_div(n_def * 32, 256)), 256, 0, s>>>(P, n_def);
             KERNEL_CHECK();
@@ -628,6 +665,7 @@ void run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, unsigned long
     }
     CUDA_CHECK(cudaMemcpyAsync(h_ctr, P.counters, sizeof(unsigned long long) * CTR_COUNT, cudaMemcpyDeviceToHost, s));
     CUDA_CHECK(cudaStreamSynchronize(s));
+    return n_keys;
 }
 
 template <typename IdxT>
@@ -654,13 +692,14 @@ void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
     P.out_lo = out_lo.p; P.out_raw = out_raw.p; P.out_surv = out_surv.p; P.proc_bits = A.bits.p; P.counters = counters.p;
     unsigned long long h_ctr[CTR_COUNT];
     ctx->t_probe.begin();
-    run_probe_kernels<IdxT>(ctx, P, h_ctr);
+    const u64 n_keys = run_probe_kernels<IdxT>(ctx, P, plan.mode, h_ctr);
     ctx->t_probe.end(1, h_ctr[CTR_ALG_BYTES]);
     ctx->st.n_probes += np;
     ctx->st.n_searched += h_ctr[CTR_SEARCHED];
     ctx->st.n_skipped_n += h_ctr[CTR_SKIP_N];
     ctx->st.n_skipped_card += h_ctr[CTR_SKIP_CARD];
     ctx->st.n_matches += h_ctr[CTR_MATCHES];
+    ctx->n_probe_keys += n_keys;
 
     // match offsets + event list + emission, fused into one scan
     ctx->t_emit.begin();
@@ -1139,6 +1178,7 @@ const char* asgart_b200_ctx_last_error(const asgart_b200_ctx* ctx) { return ctx 
 int32_t asgart_b200_ctx_set_index_bits(asgart_b200_ctx* ctx, int32_t bits) {
     if (!ctx || (bits != 0 && bits != 32 && bits != 64)) return ASGART_B200_EINVAL;
     ctx->want_bits = bits;
+    drop_sorted_keys(ctx);
     return ASGART_B200_OK;
 }
 
@@ -1146,6 +1186,7 @@ int32_t asgart_b200_ctx_load_strand(asgart_b200_ctx* ctx, const uint8_t* T, int6
     return guarded(ctx, [&]() -> int32_t {
         if (!T || n_plus_1 < 1) return fail(ctx, ASGART_B200_EINVAL, "null strand or n_plus_1 < 1");
         ctx->have_strand = ctx->have_index = false;
+        drop_sorted_keys(ctx);
         ctx->pn_mode = -1;
         ctx->n1 = u64(n_plus_1);
         EventTimer th(ctx->stream);
@@ -1178,6 +1219,7 @@ int32_t asgart_b200_ctx_load_strand(asgart_b200_ctx* ctx, const uint8_t* T, int6
 int32_t asgart_b200_ctx_ingest_begin(asgart_b200_ctx* ctx) {
     return guarded(ctx, [&]() -> int32_t {
         ctx->have_strand = ctx->have_index = false;
+        drop_sorted_keys(ctx);
         ctx->pn_mode = -1;
         ctx->pieces.clear();
         ctx->ingesting = true;
@@ -1540,7 +1582,7 @@ int32_t asgart_b200_ctx_probe_ranges(asgart_b200_ctx* ctx, const asgart_b200_chu
             counters.zero();
             P.counters = counters.p;
             unsigned long long h_ctr[CTR_COUNT];
-            run_probe_kernels<IdxT>(ctx, P, h_ctr);
+            ctx->n_probe_keys += run_probe_kernels<IdxT>(ctx, P, plan.mode, h_ctr);
         };
         if (ctx->idx_bits == 32) launch(u32(0)); else launch(u64(0));
         CUDA_CHECK(cudaMemcpyAsync(lo, d_lo.p, n_probes * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1866,7 +1908,10 @@ void asgart_b200_ctx_reset_stats(asgart_b200_ctx* ctx) {
     } catch (...) {}
     ctx->launches.total = 0;
     ctx->st = asgart_b200_stats{};
+    ctx->n_probe_keys = 0;
 }
+
+uint64_t asgart_b200_ctx_probe_keys(const asgart_b200_ctx* ctx) { return ctx ? ctx->n_probe_keys : 0; }
 
 int32_t asgart_b200_ctx_timer_start(asgart_b200_ctx* ctx) {
     return guarded(ctx, [&]() -> int32_t { CUDA_CHECK(cudaEventRecord(ctx->ev_a, ctx->stream)); return ASGART_B200_OK; });

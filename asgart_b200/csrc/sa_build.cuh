@@ -539,6 +539,9 @@ struct SaKeyHook {
     virtual void on_sorted_keys(const u64* d_keys, u64 n_local, u64 base, u64 n_total, int b, int p0, const uint16_t* h_code,
                                 cudaStream_t stream, SaGroup* grp) = 0;
     virtual bool lookup_tables(SaLookupTables&) { return false; }
+    // Single-device build that looked ranks up in the sorted keys: the buffer still holds all n keys in suffix-array
+    // order when the build ends. The hook may take it (move from `keys`); what it leaves is released.
+    virtual void adopt_sorted_keys(DevBuf<u64>& keys) { (void)keys; }
     virtual ~SaKeyHook() = default;
 };
 
@@ -1053,6 +1056,10 @@ void build_suffix_array(const u8* d_text, u64 n, IdxT* d_sa, const RankView<IdxT
         H <<= 1;
     }
     if (grp && lazy) { CUDA_CHECK(cudaStreamSynchronize(stream)); grp->barrier(); }   // the peers are done reading these keys
+    // The lazy path never writes the sorted keys after the initial sort, and only one of the two buffers is left (the
+    // other went after the rank scatter). The doubling rounds only reorder suffixes inside a group of equal keys, and such a
+    // group is one contiguous range of the final suffix array, so keys[i] is still the key of SA[i].
+    if (lazy && !grp && hook) hook->adopt_sorted_keys(keysA.p ? keysA : keysB);
     keysA.release(); keysB.release();
     phase("doubling rounds", st ? st->rounds : 0);
     nv.next("sa_build/share SA pieces");

@@ -304,6 +304,11 @@ struct ProbeParams {
     const IdxT* lut_hi;
     const IdxT* deep;     // deep table: 4^deep_depth + 1 non-decreasing bucket starts, or null
     int deep_depth;
+    // the build's sorted initial keys (keys[i] = first key_p0 symbols of suffix SA[i], key_b bits each, first symbol on
+    // top) and the map strand code -> key code (one nibble per CODE_*); null: deep buckets are compared on the text
+    const u64* keys;
+    int key_b, key_p0;
+    u64 key_map;
     const u32* q6_bits;   // 5^8 bits
     const ChunkDev* chunks;
     u32 n_chunks;
@@ -387,31 +392,87 @@ __device__ __forceinline__ u64 probe_literal(const ProbeParams<IdxT>& P, u64 q, 
     return rstart - lstart;
 }
 
+// The block's counts go to the counters with one atomic per counter: same-address atomics serialise in one L2 slice, and
+// with one per warp and counter they bounded this kernel once the keys had shortened the search (on B200 at C4 size, one
+// more per-warp counter took the keys comparison from 44 to 59 ms). Every thread of the block calls this (it synchronises
+// the block); blockDim.x == 256.
 template <typename IdxT>
 __device__ __forceinline__ void probe_account(const ProbeParams<IdxT>& P, const ProbeState& S) {
-    const unsigned n_searched = __popc(__ballot_sync(0xffffffffu, S.searched));
-    const unsigned n_skip_n = __popc(__ballot_sync(0xffffffffu, S.skip_n));
-    const unsigned n_skip_card = __popc(__ballot_sync(0xffffffffu, S.skip_card));
-    const u64 w_surv = warp_sum_u64(S.surv);
-    const u64 w_alg = warp_sum_u64(S.alg);
+    __shared__ u64 part[8][5];
+    const u64 v[5] = {__popc(__ballot_sync(0xffffffffu, S.searched)), __popc(__ballot_sync(0xffffffffu, S.skip_n)),
+                      __popc(__ballot_sync(0xffffffffu, S.skip_card)), warp_sum_u64(S.surv), warp_sum_u64(S.alg)};
     if (lane_id() == 0) {
-        if (n_searched) atomicAdd(&P.counters[CTR_SEARCHED], (unsigned long long)n_searched);
-        if (n_skip_n) atomicAdd(&P.counters[CTR_SKIP_N], (unsigned long long)n_skip_n);
-        if (n_skip_card) atomicAdd(&P.counters[CTR_SKIP_CARD], (unsigned long long)n_skip_card);
-        if (w_surv) atomicAdd(&P.counters[CTR_MATCHES], (unsigned long long)w_surv);
-        if (w_alg) atomicAdd(&P.counters[CTR_ALG_BYTES], (unsigned long long)w_alg);
+#pragma unroll
+        for (int c = 0; c < 5; ++c) part[threadIdx.x >> 5][c] = v[c];
     }
+    __syncthreads();
+    if (threadIdx.x < 5) {
+        u64 sum = 0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) sum += part[w][threadIdx.x];
+        const int ctr[5] = {CTR_SEARCHED, CTR_SKIP_N, CTR_SKIP_CARD, CTR_MATCHES, CTR_ALG_BYTES};
+        if (sum) atomicAdd(&P.counters[ctr[threadIdx.x]], (unsigned long long)sum);
+    }
+}
+
+// equal range of a deep bucket [lo0, lo0 + B) from the sorted keys: keys[lo0 ..] are compared with the probe's first
+// m = min(k, p0) symbols, and only suffixes whose key equals them, when k > p0, are compared on the text (cmp_kmer).
+// The bucket holds none of the last k-1 suffixes, so the m compared symbols of every key are text symbols (a '$' among
+// them already differs from the probe, which has none): the key comparison is the text comparison of those m symbols.
+template <typename IdxT, int kProbeLinear>
+__device__ __forceinline__ void probe_keys(const ProbeParams<IdxT>& P, u64 lo0, u64 B, u64 q, const Win& pw_raw, const Win& pw0,
+                                           ProbeState& S) {
+    const int k = int(P.k), b = P.key_b, p0 = P.key_p0;
+    const int m = k < p0 ? k : p0;
+    u64 pk = 0;   // the probe's first m symbols as a key (every needle symbol has a key code: run_probe_kernels)
+    for (int j = 0; j < m; ++j) {
+        const u32 sym = u32((j < 16 ? pw_raw.hi : pw_raw.lo) >> (60 - 4 * (j & 15))) & 15u;
+        pk = (pk << b) | ((P.key_map >> (4 * sym)) & 15u);
+    }
+    const int sh = b * (p0 - m);
+    const u64* __restrict__ K = P.keys + lo0;
+    u64 r0, r1;
+    if (B <= kProbeLinear) {
+        u64 kv[kProbeLinear];
+#pragma unroll
+        for (int j = 0; j < kProbeLinear; ++j) kv[j] = u64(j) < B ? K[j] : 0;
+        u32 lt = 0, le = 0;
+#pragma unroll
+        for (int j = 0; j < kProbeLinear; ++j) {
+            const u64 v = kv[j] >> sh;
+            if (u64(j) < B) { lt += v < pk; le += v <= pk; }
+        }
+        r0 = lt; r1 = le;
+        if (k > p0 && r1 > r0) {   // keys equal to the probe's on [r0, r1): the k-mers there run smaller, equal, greater
+            u64 lo = r0, hi = r1;
+#pragma unroll 1
+            for (u64 j = r0; j < r1; ++j) {
+                const int c = cmp_kmer(P.PT, u64(P.SA[lo0 + j]), P.PN, q, k, pw0);
+                if (c > 0) { hi = j; break; }
+                lo += c < 0;
+            }
+            r0 = lo; r1 = hi;
+        }
+    } else {
+        equal_range_lockstep(B, [&](u64 ix) -> int {
+            const u64 v = K[ix] >> sh;
+            if (v != pk) return v < pk ? -1 : 1;
+            return k > p0 ? cmp_kmer(P.PT, u64(P.SA[lo0 + ix]), P.PN, q, k, pw0) : 0;
+        }, r0, r1);
+    }
+    S.lo = lo0 + r0; S.hi = lo0 + r1;
 }
 
 // deep buckets up to LINEAR suffixes are compared in one go instead of bisected (template parameter of the kernel)
 
 // One lane per probe position. Probes whose first deep_depth bases are all ACGT start from the deep table's bucket
 // (a few suffixes) and compare them all at once; the equal range of a monotone comparator does not depend on how it is
-// searched, so this is the reference's answer whenever its own 8-mer bucket holds none of the last k-1 suffixes. Every
-// other probe (N among the first bases, flagged bucket, no deep table) takes probe_literal, in this kernel when
-// P.deferred is null and in probe_deferred_kernel otherwise (keeps the long bisections out of the short warps); probes
-// with long match intervals leave the filter pass to that kernel as well.
-template <typename IdxT, int kProbeLinear, int MINB>
+// searched, so this is the reference's answer whenever its own 8-mer bucket holds none of the last k-1 suffixes. KEYS:
+// the bucket is compared in the sorted initial keys (probe_keys), else on the text through SA. Every other probe (N among
+// the first bases, flagged bucket, no deep table) takes probe_literal, in this kernel when P.deferred is null and in
+// probe_deferred_kernel otherwise (keeps the long bisections out of the short warps); probes with long match intervals
+// leave the filter pass to that kernel as well. The keys only come with a deep table, so KEYS always defers.
+template <typename IdxT, int kProbeLinear, int MINB, bool KEYS>
 __global__ void __launch_bounds__(256, MINB) probe_search_kernel(const ProbeParams<IdxT> P) {
     const u64 g = P.p_begin + u64(blockIdx.x) * blockDim.x + threadIdx.x;
     const bool in_range = g < P.p_end;
@@ -437,7 +498,9 @@ __global__ void __launch_bounds__(256, MINB) probe_search_kernel(const ProbePara
             const u64* __restrict__ PT = P.PT;
             const u64* __restrict__ PN = P.PN;
             const u64 B = hi0 - lo0;
-            if (B <= kProbeLinear) {
+            if constexpr (KEYS) {
+                probe_keys<IdxT, kProbeLinear>(P, lo0, B, q, pw_raw, pw0, S);
+            } else if (B <= kProbeLinear) {
                 u64 xs[kProbeLinear];
 #pragma unroll
                 for (int j = 0; j < kProbeLinear; ++j) xs[j] = u64(j) < B ? u64(sub[j]) : 0;
@@ -460,7 +523,7 @@ __global__ void __launch_bounds__(256, MINB) probe_search_kernel(const ProbePara
                 S.lo = lo0 + r0; S.hi = lo0 + r1;
             }
             if (!probe_finish(P, ch, g, i, bucket8, P.deferred != nullptr, S)) defer = g | kDeferRange;
-        } else if (P.deferred) {
+        } else if (KEYS || P.deferred) {
             defer = g | (u64(1) << 62);  // bit 62 only marks the entry as present (g may be 0)
         } else {
             const u64 bucket8 = probe_literal(P, q, pw_raw, S);

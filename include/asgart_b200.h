@@ -267,6 +267,10 @@ typedef struct asgart_b200_stats {
 } asgart_b200_stats;
 ASGART_B200_API int32_t asgart_b200_ctx_stats(const asgart_b200_ctx *ctx, asgart_b200_stats *out);
 ASGART_B200_API void asgart_b200_ctx_reset_stats(asgart_b200_ctx *ctx);
+/* probes of search and probe_ranges calls since the last reset_stats whose equal range came from the sorted initial keys
+ * that a single-device build_index keeps with the index, instead of from suffix-array entries and text windows
+ * (0 for a null context) */
+ASGART_B200_API uint64_t asgart_b200_ctx_probe_keys(const asgart_b200_ctx *ctx);
 /* a CUDA-event stopwatch on the library's stream, for timing a region of calls on the device */
 ASGART_B200_API int32_t asgart_b200_ctx_timer_start(asgart_b200_ctx *ctx);
 ASGART_B200_API int32_t asgart_b200_ctx_timer_stop(asgart_b200_ctx *ctx, double *elapsed_ms);
