@@ -85,7 +85,6 @@ struct asgart_b200_ctx {
     bool group_owned = false;
     void* rank_slice = nullptr;
     size_t rank_slice_bytes = 0;
-    MemberScratch scratch;    // exchange buffers of the sharded build that the peers map
     std::vector<void*> retired_slices;
     // GPU-side FASTA ingest: one piece per file between ingest_begin and ingest_finish; pinned staging for ingest_file
     bool ingesting = false;
@@ -271,11 +270,12 @@ struct LutHook : SaKeyHook {
             const u32 code = code_of_byte(u8(*c)), dense = h_code[u8(*c)];
             if (dense && dense < 16) ix.key_map = (ix.key_map & ~(u64(15) << (4 * code))) | (u64(dense) << (4 * code));
         }
-        // depth: buckets of a few suffixes (4^depth <= n), at most 15 symbols (4 GiB of u32 starts: buckets of ~3 suffixes
-        // for a 3.1 Gbp strand, which one round of parallel loads compares, instead of a bisection), inside the initial key
-        static const int depth_cap = std::min(15, getenv("ASGART_B200_DEEP_MAX") ? atoi(getenv("ASGART_B200_DEEP_MAX")) : 15);
+        // depth: buckets of a few suffixes (4^depth <= n), inside the initial key, at most kMaxDepth symbols: 4^15 + 1 slots
+        // still fit u32 slot arithmetic (4 GiB of u32 starts), and a 3.1 Gbp strand leaves ~3 suffixes per bucket, which one
+        // round of parallel loads compares instead of a bisection
+        constexpr int kMaxDepth = 15;
         int depth = 0;
-        while (depth < depth_cap && depth < p0 && (u64(1) << (2 * (depth + 1))) <= n) ++depth;
+        while (depth < kMaxDepth && depth < p0 && (u64(1) << (2 * (depth + 1))) <= n) ++depth;
         if (depth < 4) depth = 0;
         ix.lut_lo.alloc(kLutSize, stream);
         ix.lut_hi.alloc(kLutSize, stream);
@@ -356,9 +356,8 @@ struct LutHook : SaKeyHook {
             const IdxT n1v = IdxT(n);
             CUDA_CHECK(cudaMemcpyAsync(dp + (M - 1), &n1v, sizeof(IdxT), cudaMemcpyHostToDevice, stream));
             // short empty runs (the rule in a genome-sized table) in one pass; a run past the look-ahead leaves the rest to the scan
-            static const bool fill_scan_only = getenv("ASGART_B200_DEEP_FILL") && getenv("ASGART_B200_DEEP_FILL")[0] == 's';   // developer knob: "scan"
-            u32 h_over = 1;
-            if (!fill_scan_only) {
+            u32 h_over = 0;
+            {
                 DevBuf<u32> d_over(1, stream);
                 d_over.zero();
                 deep_fill_kernel<IdxT><<<kNumSMs * 16, 256, 0, stream>>>(dp, M, d_over.p);
@@ -409,7 +408,6 @@ void build_index_t(asgart_b200_ctx* ctx) {
             CUDA_CHECK(cudaMalloc(&ctx->rank_slice, need));
             ctx->rank_slice_bytes = need;
         }
-        grp->scratch = &ctx->scratch;
         void* all[kMaxWorld] = {};
         grp->exchange_ptr(ctx->rank_slice, ctx->rank_slice_bytes, all);
         for (int r = 0; r < kMaxWorld; ++r) rv.base[r] = static_cast<IdxT*>(all[r < grp->world ? r : 0]);
@@ -879,7 +877,7 @@ void run_stage_b(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
         }
         // automaton
         DevBuf<i64> op_target(n_matches, s);
-        DevBuf<u64> a_ls(n_matches, s), a_le(n_matches, s), a_rs(n_matches, s), a_re(n_matches, s), a_death(n_matches, s);
+        DevBuf<u64> a_ls(n_matches, s), a_le(n_matches, s), a_rs(n_matches, s), a_re(n_matches, s);
         DevBuf<u32> act_arm(n_matches, s);
         DevBuf<u64> act_wlo(n_matches, s), act_whi(n_matches, s), act_death(n_matches, s), act_ls(n_matches, s);
         DevBuf<asgart_b200_protosd> out_sd(n_matches, s);
@@ -888,20 +886,16 @@ void run_stage_b(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
         AutoBuffers B{};
         B.ev_i = ev_i.p; B.ev_t = ev_t.p; B.ev_moff = ev_moff; B.ev_cnt = ev_cnt; B.ev_chunk = ev_chunk.p;
         B.seg_first = seg_first.p; B.matches = matches; B.op_target = op_target.p;
-        B.a_ls = a_ls.p; B.a_le = a_le.p; B.a_rs = a_rs.p; B.a_re = a_re.p; B.a_death = a_death.p;
+        B.a_ls = a_ls.p; B.a_le = a_le.p; B.a_rs = a_rs.p; B.a_re = a_re.p;
         B.act_arm = act_arm.p; B.act_ls = act_ls.p; B.act_wlo = act_wlo.p; B.act_whi = act_whi.p; B.act_death = act_death.p;
         B.out_sd = out_sd.p; B.out_flag = out_flag.p; B.chunk_tc = tc.p; B.chunks = plan.dev.p;
-        if (getenv("ASGART_B200_AUTOMATON_V1"))  // thread-per-segment reference kernel, kept for A/B checks
-            automaton_kernel<<<unsigned(ceil_div(n_seg, 64)), 64, 0, s>>>(B, plan.ap, n_seg, st->reverse ? 1 : 0, st->complement ? 1 : 0);
-        else {
-            // light segments: one warp each; heavy segments: one 8-warp block each (every block checks which launch owns it)
-            automaton_segment_kernel<1, kActCapLight><<<unsigned(n_seg), 32, 0, s>>>(B, plan.ap, n_seg, n_matches, n_events,
-                                                                                     st->reverse ? 1 : 0, st->complement ? 1 : 0);
-            KERNEL_CHECK();
-            automaton_segment_kernel<kHeavyWarps, kActCapHeavy><<<unsigned(n_seg), kHeavyWarps * 32, 0, s>>>(
-                B, plan.ap, n_seg, n_matches, n_events, st->reverse ? 1 : 0, st->complement ? 1 : 0);
-            count_launch();
-        }
+        // light segments: one warp each; heavy segments: one 8-warp block each (every block checks which launch owns it)
+        automaton_segment_kernel<1, kActCapLight><<<unsigned(n_seg), 32, 0, s>>>(B, plan.ap, n_seg, n_matches, n_events,
+                                                                                 st->reverse ? 1 : 0, st->complement ? 1 : 0);
+        KERNEL_CHECK();
+        automaton_segment_kernel<kHeavyWarps, kActCapHeavy><<<unsigned(n_seg), kHeavyWarps * 32, 0, s>>>(
+            B, plan.ap, n_seg, n_matches, n_events, st->reverse ? 1 : 0, st->complement ? 1 : 0);
+        count_launch();
         KERNEL_CHECK();
         count_launch();
         // compaction into CSR families
@@ -1159,7 +1153,6 @@ void asgart_b200_ctx_destroy(asgart_b200_ctx* ctx) {
     ctx->group = nullptr;
     if (ctx->rank_slice) cudaFree(ctx->rank_slice);
     for (void* p : ctx->retired_slices) cudaFree(p);
-    ctx->scratch.release();
     ctx->pieces.clear();
     for (int i = 0; i < 2; ++i) {
         if (ctx->stage[i]) cudaFreeHost(ctx->stage[i]);

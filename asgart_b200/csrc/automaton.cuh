@@ -52,7 +52,7 @@ struct AutoBuffers {
     const u64* seg_first;  // n_segments + 1 entries (last = n_events)
     const u64* matches;
     i64* op_target;
-    u64 *a_ls, *a_le, *a_rs, *a_re, *a_death;  // arm store, indexed like matches
+    u64 *a_ls, *a_le, *a_rs, *a_re;  // arm store, indexed like matches
     // active list of the warp kernel (arms that can still be extended), same capacity, creation order preserved
     u32* act_arm;   // index into the segment's arm store
     u64* act_ls;
@@ -64,30 +64,6 @@ struct AutoBuffers {
     const u64* chunk_tc;                       // processed iterations per chunk
     const ChunkDev* chunks;
 };
-
-// v1: one thread per segment (the simulation is sequential in its events; segments are independent)
-__global__ void automaton_kernel(AutoBuffers B, AutoParams P, u64 n_segments, u32 reversed_flag, u32 complemented_flag) {
-    const u64 sidx = u64(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (sidx >= n_segments) return;
-    const u64 e0 = B.seg_first[sidx], e1 = B.seg_first[sidx + 1];
-    const u32 c = B.ev_chunk[e0];
-    const ChunkDev ch = B.chunks[c];
-    const u64 slot0 = B.ev_moff[e0];
-    ArmStore arms{B.a_ls + slot0, B.a_le + slot0, B.a_rs + slot0, B.a_re + slot0, B.a_death + slot0};
-    u64 cursor = slot0;
-    simulate_segment(e0, e1, B.ev_i, B.ev_t, B.ev_moff, B.ev_cnt, B.matches, B.op_target, arms, P, ch.c0, ch.len,
-                     B.chunk_tc[c], [&](const SdOut& sd, bool head) {
-                         asgart_b200_protosd o;
-                         o.left = sd.left; o.right = sd.right;
-                         o.left_length = sd.left_length; o.right_length = sd.right_length;
-                         o.identity = 0.f;
-                         o.reversed = u8(reversed_flag); o.complemented = u8(complemented_flag);
-                         o._pad[0] = o._pad[1] = 0;
-                         B.out_sd[cursor] = o;
-                         B.out_flag[cursor] = head ? 3 : 1;
-                         ++cursor;
-                     });
-}
 
 // One warp per segment. Same event-driven semantics as simulate_segment (automaton_core.h), with the work of one
 // event spread over the lanes:

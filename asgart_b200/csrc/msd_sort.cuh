@@ -530,7 +530,7 @@ __device__ __forceinline__ u32 msd_sub_off(const u32* cnt, u32 sub) { return (cn
 template <typename IdxT, typename OffT>
 __device__ void msd_local_sort_range(const u64* __restrict__ src_k, const IdxT* __restrict__ src_v, u64* __restrict__ dst_k,
                                      IdxT* __restrict__ dst_v, u64 lo, u32 count, const OffT* __restrict__ E, u32 ba, u32 bb,
-                                     int shift, u32 dmask, u64* sk, IdxT* sv, unsigned char* aux, bool allow_fast) {
+                                     int shift, u32 dmask, u64* sk, IdxT* sv, unsigned char* aux) {
     __shared__ u32 wsm[32];
     __shared__ u32 s_max;
     const u32 tid = threadIdx.x;
@@ -570,7 +570,7 @@ __device__ void msd_local_sort_range(const u64* __restrict__ src_k, const IdxT* 
     // w = key bits of the in-smem partition step: as many as the counters allow for this many children
     int w = 0;
     while (w < 12 && w < shift && (u64(nchild) << (w + 1)) <= u64(kLocCounters)) ++w;
-    const bool fast = allow_fast && nchild >= 1 && nchild <= u32(kLocCounters) && shift > 0;
+    const bool fast = nchild >= 1 && nchild <= u32(kLocCounters) && shift > 0;
     const u32 nsub = fast ? (nchild << w) : 0;
     for (u32 i = tid; i <= nsub / 2; i += kLocThreads) cnt[i] = 0;
     if (tid == 0) s_max = 0;
@@ -770,7 +770,7 @@ template <typename IdxT, typename OffT>
 __global__ void __launch_bounds__(kLocThreads, 2)
 msd_local_kernel(const u64* __restrict__ src_k, const IdxT* __restrict__ src_v, u64* __restrict__ dst_k, IdxT* __restrict__ dst_v,
                  const OffT* __restrict__ table, const MsdBatch* __restrict__ batches, const u32* __restrict__ n_batches, int shift,
-                 u32 dmask, int allow_fast) {
+                 u32 dmask) {
     extern __shared__ __align__(16) unsigned char msd_smem[];
     u64* sk = reinterpret_cast<u64*>(msd_smem);
     IdxT* sv = reinterpret_cast<IdxT*>(sk + kLocCap);
@@ -778,7 +778,7 @@ msd_local_kernel(const u64* __restrict__ src_k, const IdxT* __restrict__ src_v, 
     if (blockIdx.x >= *n_batches) return;
     const MsdBatch bt = batches[blockIdx.x];
     msd_local_sort_range<IdxT, OffT>(src_k, src_v, dst_k, dst_v, bt.lo, bt.count, table + u64(bt.row) * kMsdBins, bt.ba, bt.bb, shift, dmask,
-                                     sk, sv, aux, allow_fast != 0);
+                                     sk, sv, aux);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -817,7 +817,6 @@ bool msd_sort_suffixes(const u8* d_text, u64 n, const uint16_t* d_code, int b, i
         CUDA_CHECK(cudaFuncSetAttribute(msd_local_kernel<IdxT, OffT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_loc)));
         device_prepared(prepared, dev_bit);
     }
-    static const bool local_fast = !(getenv("ASGART_B200_MSD_LOCAL") && getenv("ASGART_B200_MSD_LOCAL")[0] == 's');   // developer knob: "slow"
     DevBuf<unsigned long long> d_ctr(2, stream);
     DevBuf<u32> d_err(1, stream);
     d_err.zero();
@@ -937,7 +936,7 @@ bool msd_sort_suffixes(const u8* d_text, u64 n, const uint16_t* d_code, int b, i
                 msd_batches_kernel<OffT><<<unsigned(ceil_div(wins_ub, 8)), 256, 0, stream>>>(tp, win_desc.p, n_wins, batches.p, n_batches.p, u32(cap), d_err.p);
                 KERNEL_CHECK();
                 msd_local_kernel<IdxT, OffT><<<unsigned(cap), kLocThreads, smem_loc, stream>>>(dst_k, dst_v, keys_a, vals_a, tp, batches.p, n_batches.p,
-                                                                                              shift, dmask, local_fast ? 1 : 0);
+                                                                                              shift, dmask);
                 KERNEL_CHECK();
                 count_launch(2);
                 if (st && st->local) st->local->end(1, (elems - h_ctr[1]) * 2 * (sizeof(u64) + sizeof(IdxT)));

@@ -13,8 +13,8 @@
 //   2. group heads by key change (hp_reduce / hp_emit) -> SA[] for all; suffixes in groups of size > 1 are compacted into
 //      the work list (G = group head index, I = suffix), those whose p0 symbols are all equal into the run round's list.
 //      rank[] (= SA index of the group head) is NOT materialised after the MSD sort: it starts as a sentinel and a gather
-//      that meets the sentinel looks the initial rank up in the sorted keys (initial_rank below: "lazy ranks"); the LSD
-//      path and ASGART_B200_LAZY_RANK=0 write rank[SA[i]] = head(i) for every i (scatter.cuh).
+//      that meets the sentinel looks the initial rank up in the sorted keys (initial_rank below: "lazy ranks"); builds
+//      without lookup tables write rank[SA[i]] = head(i) for every i (scatter.cuh).
 //   3. run round: runs of >= p0 equal symbols (N-runs) ordered by (symbol after the run, run length) in one sort.
 //   4. doubling rounds h = p0, 2p0, ...: key2 = rank[I + h] + 1 (0 past the end)  [random gather],
 //      segmented sort of the work list by (G, key2), re-rank, write SA for suffixes that became unique, drop them,
@@ -603,12 +603,8 @@ void build_suffix_array(const u8* d_text, u64 n, IdxT* d_sa, const RankView<IdxT
     // That rule prices an LSD sort, where every 8 key bits are a pass over all pairs. The MSD sort moves a pair once per level
     // only while its bucket is still large, so longer keys cost it next to nothing — and every chance collision they remove is
     // a suffix the doubling rounds never see (3.1 Gbp of DNA: 18 symbols leave 4.4 % of the suffixes with a random twin, 21
-    // leave 0.07 %). So: as many symbols as 63 bits hold (all-ones stays free for padding keys). ASGART_B200_P0=formula
-    // keeps the LSD rule for A/B runs.
-    {
-        static const char* p0_knob = getenv("ASGART_B200_P0");
-        if (msd_sort_applicable(b, p0, n) && !(p0_knob && p0_knob[0] == 'f')) p0 = std::max(p0, std::min(63 / b, 32));
-    }
+    // leave 0.07 %). So: as many symbols as 63 bits hold (all-ones stays free for padding keys).
+    if (msd_sort_applicable(b, p0, n)) p0 = std::max(p0, std::min(63 / b, 32));
     DevBuf<uint16_t> d_code(256, stream);
     CUDA_CHECK(cudaMemcpyAsync(d_code.p, h_code, sizeof h_code, cudaMemcpyHostToDevice, stream));
     u64 rep_unit = 0;  // sum of 2^(b*j): a key whose p0 symbols are all equal to c is c * rep_unit
@@ -745,10 +741,9 @@ void build_suffix_array(const u8* d_text, u64 n, IdxT* d_sa, const RankView<IdxT
         if (hook) hook->on_sorted_keys(k, n_loc, base, n, b, p0, h_code, stream, grp);
         phase("lookup tables");
         {
-            static const bool lazy_off = getenv("ASGART_B200_LAZY_RANK") && getenv("ASGART_B200_LAZY_RANK")[0] == '0';   // developer knob
             SaLookupTables lt;
             // (every member of a group takes the same decision: it depends on n, the alphabet and the key length only)
-            if (!lazy_off && hook && hook->lookup_tables(lt) && lt.depth > 0 && p0 >= 8 && (!grp || b * std::min(p0, 4) >= 8)) {
+            if (hook && hook->lookup_tables(lt) && lt.depth > 0 && p0 >= 8 && (!grp || b * std::min(p0, 4) >= 8)) {
                 lazy = true;
                 rl.world = u32(world);
                 if (grp) {
@@ -834,7 +829,7 @@ void build_suffix_array(const u8* d_text, u64 n, IdxT* d_sa, const RankView<IdxT
             }
         }
         else if (!grp) inverse_scatter<IdxT>(d_sa, rpos, n, d_rank.base[0], n, stream, k, ka);
-        else if (!sharded_inverse_scatter<IdxT>(sa_loc, rpos, n_loc, n, d_rank, grp, stream) && n_loc) {
+        else if (n_loc) {   // group build without a deep table (texts under 256 symbols): plain stores through the view
             const unsigned grid = unsigned(std::min<u64>(ceil_div(n_loc, 256), u64(kNumSMs) * 16));
             scatter_view_kernel<IdxT><<<grid, 256, 0, stream>>>(sa_loc, rpos, n_loc, d_rank);
             KERNEL_CHECK();

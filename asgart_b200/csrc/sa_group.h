@@ -19,31 +19,8 @@ namespace ab200 {
 
 constexpr int kMaxWorld = 16;
 
-// Device blocks of one member that outlive a build (the peers keep them mapped): grow-only, freed with their owner.
-struct MemberScratch {
-    static constexpr int kSlots = 2;
-    void* p[kSlots] = {};
-    size_t bytes[kSlots] = {};
-    void* retired[64] = {};
-    int n_retired = 0;
-    void* get(int slot, size_t need) {
-        if (need <= bytes[slot]) return p[slot];
-        if (p[slot] && n_retired < 64) retired[n_retired++] = p[slot];   // peers may still have it mapped (CUDA IPC)
-        p[slot] = nullptr; bytes[slot] = 0;
-        if (cudaMalloc(&p[slot], need) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        bytes[slot] = need;
-        return p[slot];
-    }
-    void release() {
-        for (int i = 0; i < kSlots; ++i) { if (p[i]) cudaFree(p[i]); p[i] = nullptr; bytes[i] = 0; }
-        for (int i = 0; i < n_retired; ++i) cudaFree(retired[i]);
-        n_retired = 0;
-    }
-};
-
 struct SaGroup {
     int rank = 0, world = 1;
-    MemberScratch* scratch = nullptr;   // set by the member's context before a build
     // Sum of host values over the members. Every member calls it after synchronising its stream, so when it returns all
     // device work issued before it — on every member, including stores into peer memory — is complete and visible.
     virtual void allreduce_sum_host(uint64_t* vals, int n) = 0;
@@ -58,9 +35,9 @@ struct SaGroup {
 };
 
 // Rank array of the suffix-array build, one contiguous slice per member. Positions come in regions of 2^g (at most 256
-// regions; g >= 16), member r owns regions [r k, (r + 1) k), k = ceil(regions / world): slices are balanced to one region
-// and the inverse scatter can route (position, rank) pairs to their owners by the leading digit of the position
-// (sharded_inverse_scatter, scatter.cuh). world == 1 is the plain array.
+// regions; g >= 16), member r owns regions [r k, (r + 1) k), k = ceil(regions / world): slices are balanced to one region,
+// and ptr() finds a position's owner with a shift and a 32-bit divide (every rank store and gather of the build goes
+// through it). world == 1 is the plain array.
 template <typename IdxT>
 struct RankView {
     IdxT* base[kMaxWorld];
@@ -80,7 +57,7 @@ struct RankView {
         v.k = 1;
         return v;
     }
-    // region shift: the leading 8-bit digit of a position above 16-bit buckets (what the sort-back scatter partitions by)
+    // region shift: at most 256 regions of at least 2^16 positions
     static uint32_t pick_g(uint64_t n) {
         int bits = 0;
         for (uint64_t v = n ? n - 1 : 0; v; v >>= 1) ++bits;

@@ -1,7 +1,6 @@
 // scatter.cuh — out[idx[i]] = val[i] for an injective idx: the inverse-permutation scatter that turns "rank by sorted
-// position" into "rank by text position" in the suffix-array build. Since round 2 the build only comes here when the lazy
-// ranks of sa_build.cuh do not apply (LSD-sorted inputs — short texts, wide alphabets —, no deep table,
-// ASGART_B200_LAZY_RANK=0).
+// position" into "rank by text position" in the suffix-array build. The build only comes here when it has no lookup tables
+// for the lazy ranks of sa_build.cuh: the divsufsort64 drop-in, --trim, and texts under 256 symbols.
 //
 // A plain scatter of 4-byte values to random addresses costs a DRAM read-modify-write per element (B200, measured with
 // tools/scatter_bench.cu: 30.8 G elem/s for 57 M targets, 22.7 G elem/s for 1 G). When all targets of a launch fall
@@ -22,11 +21,8 @@
 //                                  followed by an in-order scatter into L2-sized slices (profiles/r1_scatter_bench.log):
 //                                  the L2 takes 26-51 G scattered elem/s only.
 #pragma once
-#include <vector>
-
 #include "common.cuh"
 #include "radix_sort.cuh"
-#include "sa_group.h"
 
 namespace ab200 {
 
@@ -265,136 +261,6 @@ void inverse_scatter(const IdxT* idx, const IdxT* val, u64 n, IdxT* out, u64 out
         KERNEL_CHECK();
     }
     count_launch(sweeps);
-}
-
-// ---- sharded build: rank[SA[i]] = value where rank[] is sliced over the members (RankView) -----------------------
-// Every member holds (position, value) pairs for the suffixes of ITS piece of the suffix array; the positions are spread
-// over all members' slices. Plain stores through the view are 4-byte writes over NVLink (measured: 133 ms per member at
-// two GPUs for 1.5 G pairs, against 74 ms for the whole single-GPU scatter). Instead the pairs travel in bulk:
-//   1. each member partitions its pairs by the leading digit of the position (regions of 2^g positions; a member's slice of
-//      rank[] is a whole number of regions, RankView),
-//   2. the members exchange their region counts (one small host all-reduce) — a permutation fills every region exactly,
-//      so each (sender, region) run has a fixed place in the owner's receive buffer,
-//   3. one kernel copies the runs into the owners' buffers (coalesced stores into peer memory, whole lines over NVLink),
-//   4. after a barrier every owner finishes locally: the remaining partition passes inside its regions and the
-//      per-bucket shared-memory scatter into its own slice (the tail of inverse_permutation_scatter).
-struct PeerU32 {
-    u32* p[kMaxWorld];
-};
-
-__global__ void pt_bin_starts_kernel(const u32* __restrict__ offs, u64 tiles, u32 n, u32* __restrict__ out) {
-    out[threadIdx.x] = offs[u64(threadIdx.x) * tiles];   // digit-major table of a single region: first tile of every digit
-    if (threadIdx.x == 0) out[256] = n;
-}
-
-__global__ void __launch_bounds__(256) push_pairs_kernel(const u32* __restrict__ ti, const u32* __restrict__ vi, u32 n_loc,
-                                                         const u32* __restrict__ bstart, const u64* __restrict__ pre, int g, u32 k,
-                                                         u64 slice, PeerU32 ridx, PeerU32 rval) {
-    __shared__ u32 bs[257];
-    __shared__ u64 dst0[256];   // where bin b's first pair of this member goes, relative to the owner's buffers
-    __shared__ u32 own[256];
-    for (u32 i = threadIdx.x; i < 257; i += 256) bs[i] = bstart[i];
-    {
-        const u32 b = threadIdx.x;
-        const u32 o = b / k;
-        own[b] = o < u32(kMaxWorld) ? o : 0u;
-        dst0[b] = (u64(b - o * k) << g) + pre[b];
-    }
-    __syncthreads();
-    const u64 stride = u64(gridDim.x) * blockDim.x;
-    for (u64 j = u64(blockIdx.x) * blockDim.x + threadIdx.x; j < n_loc; j += stride) {
-        u32 lo = 0, hi = 256;   // last bin with bs[bin] <= j
-        while (hi - lo > 1) { const u32 mid = (lo + hi) >> 1; if (bs[mid] <= j) lo = mid; else hi = mid; }
-        const u64 off = dst0[lo] + (j - bs[lo]);
-        if (off < slice) {
-            ridx.p[own[lo]][off] = ti[j];
-            rval.p[own[lo]][off] = vi[j];
-        }
-    }
-}
-
-// Collective over the group (every member calls it, also with n_loc == 0). Returns false — on every member alike — when
-// the shape does not fit (64-bit indices, slices shorter than a bucket): the caller then stores through the view.
-template <typename IdxT>
-bool sharded_inverse_scatter(const IdxT* idx, const IdxT* val, u64 n_loc, u64 n, const RankView<IdxT>& rv, SaGroup* grp, cudaStream_t stream) {
-    if constexpr (sizeof(IdxT) != 4) {
-        return false;
-    } else {
-        const int bits = bit_width_u64(n - 1);
-        if (bits <= kBucketBits || n >= (u64(1) << 32) || !grp->scratch) return false;
-        const int g = int(rv.g);   // leading digit = position >> g, at most 256 regions (RankView::pick_g)
-        const int world = grp->world, rank = grp->rank;
-        const u64 slice = rv.slice_len();
-        // 1. my pairs by region
-        const u64 half = (n_loc + 3) / 4 * 4;
-        DevBuf<u32> pa(2 * (half + 4), stream), hist, offs, d_bs(257, stream);
-        std::vector<u32> h_bs(257, 0);
-        if (n_loc) {
-            partition_pass(reinterpret_cast<const u32*>(idx), reinterpret_cast<const u32*>(val), n_loc, g, 0, pa.p, pa.p + half, hist, offs, stream);
-            pt_bin_starts_kernel<<<1, 256, 0, stream>>>(offs.p, ceil_div(n_loc, u64(kPtTile)), u32(n_loc), d_bs.p);
-            KERNEL_CHECK();
-            count_launch();
-            CUDA_CHECK(cudaMemcpyAsync(h_bs.data(), d_bs.p, 257 * sizeof(u32), cudaMemcpyDeviceToHost, stream));
-        } else {
-            d_bs.zero();
-        }
-        CUDA_CHECK(cudaStreamSynchronize(stream));
-        // 2. everybody's region counts -> my runs' places behind the runs of the members before me
-        std::vector<u64> all(size_t(world) * 256, 0);
-        for (int b = 0; b < 256; ++b) all[size_t(rank) * 256 + b] = u64(h_bs[b + 1]) - u64(h_bs[b]);
-        grp->allreduce_sum_host(all.data(), world * 256);
-        std::vector<u64> h_pre(256, 0);
-        for (int b = 0; b < 256; ++b)
-            for (int q = 0; q < rank; ++q) h_pre[b] += all[size_t(q) * 256 + b];
-        DevBuf<u64> d_pre(256, stream);
-        CUDA_CHECK(cudaMemcpyAsync(d_pre.p, h_pre.data(), 256 * sizeof(u64), cudaMemcpyHostToDevice, stream));
-        // 3. receive buffers (persistent: the peers map them) and the push
-        u32* recv = static_cast<u32*>(grp->scratch->get(0, 2 * slice * sizeof(u32)));
-        if (!recv) throw CudaError(ASGART_B200_ENOMEM, "sharded inverse scatter: cannot allocate the exchange buffer");
-        void* peers[kMaxWorld] = {};
-        grp->exchange_ptr(recv, 2 * slice * sizeof(u32), peers);
-        PeerU32 ridx, rval;
-        for (int r = 0; r < kMaxWorld; ++r) {
-            u32* b = static_cast<u32*>(peers[r < world ? r : 0]);
-            ridx.p[r] = b;
-            rval.p[r] = b + slice;
-        }
-        if (n_loc) {
-            const unsigned grid = unsigned(std::min<u64>(ceil_div(n_loc, 256), u64(kNumSMs) * 16));
-            push_pairs_kernel<<<grid, 256, 0, stream>>>(pa.p, pa.p + half, u32(n_loc), d_bs.p, d_pre.p, g, rv.k, slice, ridx, rval);
-            KERNEL_CHECK();
-            count_launch();
-        }
-        // 4. all runs have landed (and h_pre is no longer read by the copy above)
-        CUDA_CHECK(cudaStreamSynchronize(stream));
-        grp->barrier();
-        const u64 own0 = u64(rank) * slice;
-        const u64 n_own = own0 < n ? std::min(slice, n - own0) : 0;
-        if (n_own) {
-            const u64 ohalf = (n_own + 3) / 4 * 4;
-            DevBuf<u32> ws(g > kBucketBits ? 2 * (ohalf + 4) : 0, stream);
-            const u32 *ki = recv, *vi = recv + slice;
-            u32* bufs[2][2] = {{ws.p, ws.p + ohalf}, {recv, recv + slice}};
-            int w = 0;
-            for (int shift = g - 8; shift >= kBucketBits; shift -= 8) {
-                partition_pass(ki, vi, n_own, shift, u64(1) << (shift + 8), bufs[w][0], bufs[w][1], hist, offs, stream);
-                ki = bufs[w][0]; vi = bufs[w][1];
-                w ^= 1;
-            }
-            static std::atomic<unsigned long long> prepared{0};
-            constexpr int smem = int(sizeof(u32)) << kBucketHalfBits;
-            unsigned long long dev_bit = 0;
-            if (device_needs_prepare(prepared, dev_bit)) {
-                CUDA_CHECK(cudaFuncSetAttribute(bucket_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-                device_prepared(prepared, dev_bit);
-            }
-            bucket_scatter_kernel<<<unsigned(ceil_div(n_own, u64(1) << kBucketBits)), kBucketThreads, smem, stream>>>(ki, vi, n_own,
-                                                                                                                   reinterpret_cast<u32*>(rv.base[rank]));
-            KERNEL_CHECK();
-            count_launch();
-        }
-        return true;
-    }
 }
 
 }  // namespace ab200

@@ -199,7 +199,7 @@ void* emul_search(const uint8_t* text, int64_t n1_, const int64_t* SA, const asg
         if (head) seg_first.push_back(e);
     }
     seg_first.push_back(ne);
-    // automaton, one segment at a time (automaton_kernel)
+    // automaton, one segment at a time (simulate_segment)
     Result* R = new Result();
     const u64 nm = matches.size();
     std::vector<int64_t> op(nm);

@@ -173,26 +173,6 @@ def test_stale_keys_are_not_used(bits):
         assert got.as_lists() == oracle.search_trim(b, trim, [chunk], so, oracle.POST_ALL, threads=4).as_lists()
 
 
-_LAZY_OFF_SCRIPT = r"""
-import sys
-sys.path.insert(0, {root!r})
-from tests import cases
-from tests.test_gpu_probe_keys import _strand, run_text
-strand = _strand(cases.stress_text(5, n=50_000))
-for bits in (32, 64):
-    run_text(strand, bits, (20, 32), lambda st: False, chunk=(1000, 30_000), every=3)
-print("lazy off ok")
-"""
-
-
-def test_without_lazy_ranks_keys_are_scratch():
-    """ASGART_B200_LAZY_RANK=0: the sort-back scatter overwrites the key buffers, so nothing is kept and the text path
-    gives the same answers."""
-    env = dict(os.environ, ASGART_B200_LAZY_RANK="0")
-    r = subprocess.run([sys.executable, "-c", _LAZY_OFF_SCRIPT.format(root=ROOT)], env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "lazy off ok" in r.stdout, r.stdout + r.stderr
-
-
 def test_group_build_keeps_no_keys():
     """Members of a sharded build hold only their key range: their searches take the text path, with the families of a
     single-device build."""
