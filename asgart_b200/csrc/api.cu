@@ -52,12 +52,10 @@ struct StageA {
 
 using namespace ab200;
 
+// host copy of a shard's partial: meta = {p_begin, p_end, events, matches}, blob = the device blob's bytes (blob_layout)
 struct asgart_b200_partial {
-    u64 p_begin = 0, p_end = 0;
-    std::vector<u32> bits;
-    std::vector<u64> ev_probe;
-    std::vector<u32> ev_cnt;
-    std::vector<u64> matches;
+    u64 meta[4] = {0, 0, 0, 0};
+    std::vector<u8> blob;
 };
 
 struct asgart_b200_ctx {
@@ -106,6 +104,7 @@ struct asgart_b200_hits {
 namespace ab200 { namespace detail {
 
 const u64 kPartialMagic = 0x4132303050415254ull;  // "A200PART"
+const u64 kPartialHeader = 6 * 8;                  // serialised partial: {magic, meta[4], blob bytes}, then the blob
 
 struct ApiGuard {
     asgart_b200_ctx* c;
@@ -666,6 +665,20 @@ u64 run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, int mode, unsi
     return n_keys;
 }
 
+// the ProbeParams fields of every probe search over [p_begin, p_end) of the plan: text and needle images, index, chunks
+template <typename IdxT>
+ProbeParams<IdxT> probe_params(asgart_b200_ctx* ctx, const ChunkPlan& plan, u64 p_begin, u64 p_end) {
+    auto& ix = IxOf<IdxT>::get(ctx);
+    ProbeParams<IdxT> P{};
+    P.PT = ctx->d_pt.p;
+    P.PN = plan.mode == PACK_DIRECT ? ctx->d_pt.p : ctx->d_pn.p;
+    P.SA = ix.sa.p; P.lut_lo = ix.lut_lo.p; P.lut_hi = ix.lut_hi.p;
+    P.chunks = plan.dev.p; P.n_chunks = u32(plan.host.size());
+    P.n1 = ctx->n1; P.k = plan.k; P.s = plan.s;
+    P.p_begin = p_begin; P.p_end = p_end;
+    return P;
+}
+
 template <typename IdxT>
 void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_settings* st, u64 p_begin, u64 p_end, StageA& A) {
     NvtxRange nv("search/stage A: probe search + emit");
@@ -680,13 +693,8 @@ void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
     DevBuf<u32> out_surv(np, s);
     DevBuf<unsigned long long> counters(CTR_COUNT, s);
     counters.zero();
-    ProbeParams<IdxT> P{};
-    P.PT = ctx->d_pt.p;
-    P.PN = plan.mode == PACK_DIRECT ? ctx->d_pt.p : ctx->d_pn.p;
-    P.SA = ix.sa.p; P.lut_lo = ix.lut_lo.p; P.lut_hi = ix.lut_hi.p;
-    P.chunks = plan.dev.p; P.n_chunks = u32(plan.host.size());
-    P.n1 = ctx->n1; P.k = plan.k; P.s = plan.s; P.reverse = st->reverse ? 1 : 0; P.max_card = st->max_cardinality;
-    P.p_begin = p_begin; P.p_end = p_end;
+    ProbeParams<IdxT> P = probe_params<IdxT>(ctx, plan, p_begin, p_end);
+    P.reverse = st->reverse ? 1 : 0; P.max_card = st->max_cardinality;
     P.out_lo = out_lo.p; P.out_raw = out_raw.p; P.out_surv = out_surv.p; P.proc_bits = A.bits.p; P.counters = counters.p;
     unsigned long long h_ctr[CTR_COUNT];
     ctx->t_probe.begin();
@@ -937,6 +945,95 @@ void shard_range(u64 total, int shard, int n_shards, u64& b, u64& e) {
     if (per == 0) per = 32;
     b = std::min(total, u64(shard) * per);
     e = std::min(total, u64(shard + 1) * per);
+}
+
+// Stage A of shard `shard` of `n_shards` (ctx_search: 0 of 1): chunk plan, needle image, probe range, one index-width
+// dispatch. ms_search times stage A and whatever `in_timer` enqueues after it.
+template <typename F>
+int search_stage_a(asgart_b200_ctx* ctx, const asgart_b200_chunk* chunks, i64 n_chunks, const asgart_b200_settings* st, int shard,
+                   int n_shards, ChunkPlan& plan, StageA& A, F in_timer) {
+    if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "search before build_index");
+    int rc = make_plan(ctx, chunks, n_chunks, st, plan);
+    if (rc) return rc;
+    ensure_needle(ctx, plan.mode);
+    u64 b, e;
+    shard_range(plan.total_probes, shard, n_shards, b, e);
+    EventTimer ts(ctx->stream);
+    ts.start();
+    if (ctx->idx_bits == 32) run_stage_a<u32>(ctx, plan, st, b, e, A);
+    else run_stage_a<u64>(ctx, plan, st, b, e, A);
+    in_timer();
+    ts.stop();
+    ctx->st.ms_search += ts.ms();
+    return ASGART_B200_OK;
+}
+
+// A shard's partial, the same bytes in HBM (search_shard_dev: what an NCCL all-gather moves) and behind the header of a
+// serialised host partial (search_shard):
+//   [ processed bits (4 B x words, padded to 8) | ev_probe (8 B x events) | matches (8 B x matches) | ev_cnt (4 B x events) ]
+// meta = {p_begin, p_end, events, matches}; the section offsets and the total are in bytes.
+struct BlobLayout { u64 words, probe, matches, cnt, bytes; };
+BlobLayout blob_layout(const u64* meta) {
+    BlobLayout L;
+    L.words = ceil_div(meta[1] - meta[0], 32);
+    L.probe = ceil_div(L.words * 4, 8) * 8;
+    L.matches = L.probe + meta[2] * 8;
+    L.cnt = L.matches + meta[3] * 8;
+    L.bytes = L.cnt + meta[2] * 4;
+    return L;
+}
+
+// stage A's four arrays into their sections of a blob in device or host memory (kind); the padding is not written
+void pack_partial(const StageA& A, const BlobLayout& L, u8* blob, cudaMemcpyKind kind, cudaStream_t s) {
+    if (L.words) CUDA_CHECK(cudaMemcpyAsync(blob, A.bits.p, L.words * 4, kind, s));
+    if (A.n_events) CUDA_CHECK(cudaMemcpyAsync(blob + L.probe, A.ev_probe.p, A.n_events * 8, kind, s));
+    if (A.n_matches) CUDA_CHECK(cudaMemcpyAsync(blob + L.matches, A.matches.p, A.n_matches * 8, kind, s));
+    if (A.n_events) CUDA_CHECK(cudaMemcpyAsync(blob + L.cnt, A.ev_cnt.p, A.n_events * 4, kind, s));
+}
+
+// Stage B over the partials of all shards: device blobs and their meta words (4 per shard). The partials come from
+// other processes, so they must be the consecutive shards of this plan: 32-aligned starts, covering every probe.
+int merge_shards(asgart_b200_ctx* ctx, const asgart_b200_chunk* chunks, i64 n_chunks, const asgart_b200_settings* st,
+                 const void* const* d_blobs, const u64* metas, int n_shards, u32 post_mask, asgart_b200_result** out) {
+    if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "finish before load_strand");
+    ChunkPlan plan;
+    int rc = make_plan(ctx, chunks, n_chunks, st, plan);
+    if (rc) return rc;
+    u64 expect = 0, ne = 0, nm = 0;
+    for (int r = 0; r < n_shards; ++r) {
+        const u64 pb = metas[4 * r], pe = metas[4 * r + 1];
+        if (pb != expect || pe < pb || pe > plan.total_probes || ((pb & 31) && pb != plan.total_probes) || (!d_blobs[r] && pe > pb))
+            return fail(ctx, ASGART_B200_EINVAL, "partials are not the consecutive shards of this plan");
+        expect = pe;
+        ne += metas[4 * r + 2]; nm += metas[4 * r + 3];
+    }
+    if (expect != plan.total_probes) return fail(ctx, ASGART_B200_EINVAL, "partials do not cover all probes");
+    cudaStream_t s = ctx->stream;
+    const u64 words = ceil_div(plan.total_probes, 32);
+    DevBuf<u32> d_bits(words, s), d_cnt(ne, s);
+    DevBuf<u64> d_probe(ne, s), d_moff(ne, s), d_matches(nm, s);
+    u64 e0 = 0, m0 = 0;
+    for (int r = 0; r < n_shards; ++r) {
+        const u64* m = metas + 4 * r;
+        const BlobLayout L = blob_layout(m);
+        const u8* p = static_cast<const u8*>(d_blobs[r]);
+        if (L.words) CUDA_CHECK(cudaMemcpyAsync(d_bits.p + (m[0] >> 5), p, L.words * 4, cudaMemcpyDeviceToDevice, s));
+        if (m[2]) CUDA_CHECK(cudaMemcpyAsync(d_probe.p + e0, p + L.probe, m[2] * 8, cudaMemcpyDeviceToDevice, s));
+        if (m[3]) CUDA_CHECK(cudaMemcpyAsync(d_matches.p + m0, p + L.matches, m[3] * 8, cudaMemcpyDeviceToDevice, s));
+        if (m[2]) CUDA_CHECK(cudaMemcpyAsync(d_cnt.p + e0, p + L.cnt, m[2] * 4, cudaMemcpyDeviceToDevice, s));
+        e0 += m[2]; m0 += m[3];
+    }
+    if (ne) {
+        const u32* cp = d_cnt.p; u64* mp = d_moff.p;
+        device_scan<u64, SumOp>([cp] __device__(u64 e) { return u64(cp[e]); }, [mp] __device__(u64 e, u64 exc, u64) { mp[e] = exc; },
+                                ne, (u64*)nullptr, s);
+    }
+    asgart_b200_result* res = new asgart_b200_result();
+    try {
+        run_stage_b(ctx, plan, st, d_bits.p, ne, d_probe.p, d_cnt.p, d_moff.p, d_matches.p, nm, post_mask, res);
+    } catch (...) { delete res; throw; }
+    *out = res;
+    return ASGART_B200_OK;
 }
 
 void fold_family_timers(asgart_b200_ctx* ctx) {
@@ -1564,12 +1661,7 @@ int32_t asgart_b200_ctx_probe_ranges(asgart_b200_ctx* ctx, const asgart_b200_chu
         DevBuf<i64> d_lo(n_probes, ctx->stream), d_hi(n_probes, ctx->stream);
         auto launch = [&](auto tag) {
             using IdxT = decltype(tag);
-            auto& ix = IxOf<IdxT>::get(ctx);
-            ProbeParams<IdxT> P{};
-            P.PT = ctx->d_pt.p; P.PN = plan.mode == PACK_DIRECT ? ctx->d_pt.p : ctx->d_pn.p;
-            P.SA = ix.sa.p; P.lut_lo = ix.lut_lo.p; P.lut_hi = ix.lut_hi.p;
-            P.chunks = plan.dev.p; P.n_chunks = 1; P.n1 = ctx->n1; P.k = plan.k; P.s = plan.s;
-            P.p_begin = 0; P.p_end = u64(n_probes);
+            ProbeParams<IdxT> P = probe_params<IdxT>(ctx, plan, 0, u64(n_probes));
             P.rng_lo = d_lo.p; P.rng_hi = d_hi.p;
             DevBuf<unsigned long long> counters(CTR_COUNT, ctx->stream);
             counters.zero();
@@ -1590,18 +1682,10 @@ int32_t asgart_b200_ctx_search(asgart_b200_ctx* ctx, const asgart_b200_chunk* ch
     return guarded(ctx, [&]() -> int32_t {
         if (!out) return fail(ctx, ASGART_B200_EINVAL, "null out");
         *out = nullptr;
-        if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "search before build_index");
         ChunkPlan plan;
-        int rc = make_plan(ctx, chunks, n_chunks, st, plan);
-        if (rc) return rc;
-        ensure_needle(ctx, plan.mode);
-        EventTimer ts(ctx->stream);
-        ts.start();
         StageA A;
-        if (ctx->idx_bits == 32) run_stage_a<u32>(ctx, plan, st, 0, plan.total_probes, A);
-        else run_stage_a<u64>(ctx, plan, st, 0, plan.total_probes, A);
-        ts.stop();
-        ctx->st.ms_search += ts.ms();
+        int rc = search_stage_a(ctx, chunks, n_chunks, st, 0, 1, plan, A, [] {});
+        if (rc) return rc;
         asgart_b200_result* r = new asgart_b200_result();
         try {
             run_stage_b(ctx, plan, st, A.bits.p, A.n_events, A.ev_probe.p, A.ev_cnt.p, A.ev_moff.p, A.matches.p, A.n_matches, post_mask, r);
@@ -1616,52 +1700,28 @@ int32_t asgart_b200_ctx_search_shard(asgart_b200_ctx* ctx, const asgart_b200_chu
     return guarded(ctx, [&]() -> int32_t {
         if (!out || n_shards < 1 || shard < 0 || shard >= n_shards) return fail(ctx, ASGART_B200_EINVAL, "bad shard arguments");
         *out = nullptr;
-        if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "search before build_index");
         ChunkPlan plan;
-        int rc = make_plan(ctx, chunks, n_chunks, st, plan);
-        if (rc) return rc;
-        ensure_needle(ctx, plan.mode);
-        u64 b, e;
-        shard_range(plan.total_probes, shard, n_shards, b, e);
-        EventTimer ts(ctx->stream);
-        ts.start();
         StageA A;
-        if (ctx->idx_bits == 32) run_stage_a<u32>(ctx, plan, st, b, e, A);
-        else run_stage_a<u64>(ctx, plan, st, b, e, A);
-        ts.stop();
-        ctx->st.ms_search += ts.ms();
-        asgart_b200_partial* p = new asgart_b200_partial();
-        p->p_begin = b; p->p_end = e;
-        p->bits.resize(ceil_div(e - b, 32));
-        p->ev_probe.resize(A.n_events); p->ev_cnt.resize(A.n_events); p->matches.resize(A.n_matches);
-        cudaStream_t s = ctx->stream;
-        if (!p->bits.empty()) CUDA_CHECK(cudaMemcpyAsync(p->bits.data(), A.bits.p, p->bits.size() * 4, cudaMemcpyDeviceToHost, s));
-        if (A.n_events) {
-            CUDA_CHECK(cudaMemcpyAsync(p->ev_probe.data(), A.ev_probe.p, A.n_events * 8, cudaMemcpyDeviceToHost, s));
-            CUDA_CHECK(cudaMemcpyAsync(p->ev_cnt.data(), A.ev_cnt.p, A.n_events * 4, cudaMemcpyDeviceToHost, s));
-        }
-        if (A.n_matches) CUDA_CHECK(cudaMemcpyAsync(p->matches.data(), A.matches.p, A.n_matches * 8, cudaMemcpyDeviceToHost, s));
-        CUDA_CHECK(cudaStreamSynchronize(s));
-        ctx->st.d2h_bytes += p->bits.size() * 4 + A.n_events * 12 + A.n_matches * 8;
-        *out = p;
+        int rc = search_stage_a(ctx, chunks, n_chunks, st, shard, n_shards, plan, A, [] {});
+        if (rc) return rc;
+        std::unique_ptr<asgart_b200_partial> p(new asgart_b200_partial{{A.p_begin, A.p_end, A.n_events, A.n_matches}, {}});
+        const BlobLayout L = blob_layout(p->meta);
+        p->blob.resize(L.bytes);   // zero-filled: the padding of the processed bits is 0, as in search_shard_dev's blob
+        pack_partial(A, L, p->blob.data(), cudaMemcpyDeviceToHost, ctx->stream);
+        CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+        ctx->st.d2h_bytes += L.words * 4 + A.n_events * 12 + A.n_matches * 8;
+        *out = p.release();
         return ASGART_B200_OK;
     });
 }
 
-int64_t asgart_b200_partial_size(const asgart_b200_partial* p) {
-    if (!p) return 0;
-    return int64_t(6 * 8 + p->bits.size() * 4 + p->ev_probe.size() * 8 + p->ev_cnt.size() * 4 + p->matches.size() * 8);
-}
+int64_t asgart_b200_partial_size(const asgart_b200_partial* p) { return p ? int64_t(kPartialHeader + p->blob.size()) : 0; }
 
 int32_t asgart_b200_partial_serialize(const asgart_b200_partial* p, uint8_t* buf, int64_t cap) {
     if (!p || !buf || cap < asgart_b200_partial_size(p)) return ASGART_B200_EINVAL;
-    u64 hdr[6] = {kPartialMagic, p->p_begin, p->p_end, u64(p->bits.size()), u64(p->ev_probe.size()), u64(p->matches.size())};
-    uint8_t* w = buf;
-    memcpy(w, hdr, sizeof hdr); w += sizeof hdr;
-    memcpy(w, p->bits.data(), p->bits.size() * 4); w += p->bits.size() * 4;
-    memcpy(w, p->ev_probe.data(), p->ev_probe.size() * 8); w += p->ev_probe.size() * 8;
-    memcpy(w, p->ev_cnt.data(), p->ev_cnt.size() * 4); w += p->ev_cnt.size() * 4;
-    memcpy(w, p->matches.data(), p->matches.size() * 8);
+    const u64 hdr[6] = {kPartialMagic, p->meta[0], p->meta[1], p->meta[2], p->meta[3], u64(p->blob.size())};
+    memcpy(buf, hdr, kPartialHeader);
+    memcpy(buf + kPartialHeader, p->blob.data(), p->blob.size());
     return ASGART_B200_OK;
 }
 
@@ -1673,97 +1733,57 @@ int32_t asgart_b200_ctx_finish(asgart_b200_ctx* ctx, const asgart_b200_chunk* ch
     return guarded(ctx, [&]() -> int32_t {
         if (!out || !partials || !sizes || n_shards < 1) return fail(ctx, ASGART_B200_EINVAL, "bad finish arguments");
         *out = nullptr;
-        if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "finish before load_strand");
-        ChunkPlan plan;
-        int rc = make_plan(ctx, chunks, n_chunks, st, plan);
-        if (rc) return rc;
-        const u64 words = ceil_div(plan.total_probes, 32);
-        std::vector<u32> bits(words, 0);
-        std::vector<u64> ev_probe, matches;
-        std::vector<u32> ev_cnt;
-        u64 expect = 0;
+        // the byte format: the header, then the blob and nothing after it
+        std::vector<u64> metas(4 * size_t(n_shards)), at(size_t(n_shards) + 1, 0);   // at: the blobs' offsets in d_all
+        u64 payload = 0;
         for (int r = 0; r < n_shards; ++r) {
-            const uint8_t* b = partials[r];
-            if (!b || sizes[r] < 48) return fail(ctx, ASGART_B200_EINVAL, "partial too small");
+            if (!partials[r] || sizes[r] < i64(kPartialHeader)) return fail(ctx, ASGART_B200_EINVAL, "partial too small");
             u64 hdr[6];
-            memcpy(hdr, b, sizeof hdr);
+            memcpy(hdr, partials[r], kPartialHeader);
             if (hdr[0] != kPartialMagic) return fail(ctx, ASGART_B200_EINVAL, "bad partial magic");
-            const u64 pb = hdr[1], pe = hdr[2], nb = hdr[3], ne = hdr[4], nm = hdr[5];
-            if (pb != expect || pe < pb || pe > plan.total_probes || ((pb & 31) && pb != plan.total_probes) || nb != ceil_div(pe - pb, 32) ||
-                u64(sizes[r]) != 48 + nb * 4 + ne * 12 + nm * 8)
-                return fail(ctx, ASGART_B200_EINVAL, "partials are not the consecutive shards of this plan");
-            expect = pe;
-            const uint8_t* p = b + 48;
-            memcpy(bits.data() + (pb >> 5), p, nb * 4); p += nb * 4;
-            size_t e0 = ev_probe.size(), m0 = matches.size();
-            ev_probe.resize(e0 + ne); ev_cnt.resize(e0 + ne); matches.resize(m0 + nm);
-            memcpy(ev_probe.data() + e0, p, ne * 8); p += ne * 8;
-            memcpy(ev_cnt.data() + e0, p, ne * 4); p += ne * 4;
-            memcpy(matches.data() + m0, p, nm * 8);
+            const u64 bytes = u64(sizes[r]) - kPartialHeader;
+            const BlobLayout L = blob_layout(hdr + 1);
+            // counts the bytes could not hold are rejected first: the layout's sums do not wrap around
+            if (hdr[5] != bytes || hdr[3] > bytes / 12 || hdr[4] > bytes / 8 || L.bytes != bytes)
+                return fail(ctx, ASGART_B200_EINVAL, "partial size does not match its header");
+            std::copy(hdr + 1, hdr + 5, &metas[4 * r]);
+            at[r + 1] = at[r] + bytes;
+            payload += L.words * 4 + hdr[3] * 12 + hdr[4] * 8;
         }
-        if (expect != plan.total_probes) return fail(ctx, ASGART_B200_EINVAL, "partials do not cover all probes");
-        cudaStream_t s = ctx->stream;
-        const u64 ne = ev_probe.size(), nm = matches.size();
-        DevBuf<u32> d_bits(words, s), d_cnt(ne, s);
-        DevBuf<u64> d_probe(ne, s), d_moff(ne, s), d_matches(nm, s);
-        if (words) CUDA_CHECK(cudaMemcpyAsync(d_bits.p, bits.data(), words * 4, cudaMemcpyHostToDevice, s));
-        if (ne) {
-            CUDA_CHECK(cudaMemcpyAsync(d_probe.p, ev_probe.data(), ne * 8, cudaMemcpyHostToDevice, s));
-            CUDA_CHECK(cudaMemcpyAsync(d_cnt.p, ev_cnt.data(), ne * 4, cudaMemcpyHostToDevice, s));
-            const u32* cp = d_cnt.p; u64* mp = d_moff.p;
-            device_scan<u64, SumOp>([cp] __device__(u64 e) { return u64(cp[e]); }, [mp] __device__(u64 e, u64 exc, u64) { mp[e] = exc; },
-                                    ne, (u64*)nullptr, s);
+        DevBuf<u8> d_all(at[n_shards], ctx->stream);
+        std::vector<const void*> d_blobs(n_shards);
+        for (int r = 0; r < n_shards; ++r) {
+            d_blobs[r] = d_all.p + at[r];
+            if (at[r + 1] > at[r])
+                CUDA_CHECK(cudaMemcpyAsync(d_all.p + at[r], partials[r] + kPartialHeader, at[r + 1] - at[r], cudaMemcpyHostToDevice, ctx->stream));
         }
-        if (nm) CUDA_CHECK(cudaMemcpyAsync(d_matches.p, matches.data(), nm * 8, cudaMemcpyHostToDevice, s));
-        ctx->st.h2d_bytes += words * 4 + ne * 12 + nm * 8;
-        asgart_b200_result* r = new asgart_b200_result();
-        try {
-            run_stage_b(ctx, plan, st, d_bits.p, ne, d_probe.p, d_cnt.p, d_moff.p, d_matches.p, nm, post_mask, r);
-        } catch (...) { delete r; throw; }
-        *out = r;
-        return ASGART_B200_OK;
+        const int32_t rc = merge_shards(ctx, chunks, n_chunks, st, d_blobs.data(), metas.data(), n_shards, post_mask, out);
+        if (rc == ASGART_B200_OK) ctx->st.h2d_bytes += payload;
+        return rc;
     });
 }
-
-// Device-resident form of search_shard / finish: the partial stays in HBM as one blob
-//   [ processed bits (4 B x words, padded to 8) | ev_probe (8 B x events) | matches (8 B x matches) | ev_cnt (4 B x events) ]
-// so that the exchange is a plain NCCL all-gather of device memory (meta = {p_begin, p_end, events, matches} travels apart).
-static u64 blob_bytes_of(u64 pb, u64 pe, u64 ne, u64 nm) { return ceil_div(ceil_div(pe - pb, 32) * 4, 8) * 8 + ne * 8 + nm * 8 + ne * 4; }
 
 int32_t asgart_b200_ctx_search_shard_dev(asgart_b200_ctx* ctx, const asgart_b200_chunk* chunks, int64_t n_chunks,
                                          const asgart_b200_settings* st, int32_t shard, int32_t n_shards, void** d_blob,
                                          int64_t* blob_bytes, uint64_t* meta) {
     return guarded(ctx, [&]() -> int32_t {
         if (!d_blob || !blob_bytes || !meta || n_shards < 1 || shard < 0 || shard >= n_shards) return fail(ctx, ASGART_B200_EINVAL, "bad shard arguments");
-        if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "search before build_index");
         ChunkPlan plan;
-        int rc = make_plan(ctx, chunks, n_chunks, st, plan);
-        if (rc) return rc;
-        ensure_needle(ctx, plan.mode);
-        u64 b, e;
-        shard_range(plan.total_probes, shard, n_shards, b, e);
-        EventTimer ts(ctx->stream);
-        ts.start();
         StageA A;
-        if (ctx->idx_bits == 32) run_stage_a<u32>(ctx, plan, st, b, e, A);
-        else run_stage_a<u64>(ctx, plan, st, b, e, A);
-        cudaStream_t s = ctx->stream;
-        const u64 words = ceil_div(e - b, 32), wbytes = ceil_div(words * 4, 8) * 8;
-        const u64 total = blob_bytes_of(b, e, A.n_events, A.n_matches);
-        ctx->shard_blob.alloc(std::max<u64>(total, 8), s);
-        u8* p = ctx->shard_blob.p;
-        if (words) CUDA_CHECK(cudaMemcpyAsync(p, A.bits.p, words * 4, cudaMemcpyDeviceToDevice, s));
-        p += wbytes;
-        if (A.n_events) CUDA_CHECK(cudaMemcpyAsync(p, A.ev_probe.p, A.n_events * 8, cudaMemcpyDeviceToDevice, s));
-        p += A.n_events * 8;
-        if (A.n_matches) CUDA_CHECK(cudaMemcpyAsync(p, A.matches.p, A.n_matches * 8, cudaMemcpyDeviceToDevice, s));
-        p += A.n_matches * 8;
-        if (A.n_events) CUDA_CHECK(cudaMemcpyAsync(p, A.ev_cnt.p, A.n_events * 4, cudaMemcpyDeviceToDevice, s));
-        ts.stop();
-        ctx->st.ms_search += ts.ms();   // synchronises: the blob is complete when this call returns
-        meta[0] = b; meta[1] = e; meta[2] = A.n_events; meta[3] = A.n_matches;
+        BlobLayout L{};
+        int rc = search_stage_a(ctx, chunks, n_chunks, st, shard, n_shards, plan, A, [&] {
+            const cudaStream_t s = ctx->stream;
+            const u64 m[4] = {A.p_begin, A.p_end, A.n_events, A.n_matches};
+            L = blob_layout(m);
+            ctx->shard_blob.alloc(std::max<u64>(L.bytes, 8), s);
+            pack_partial(A, L, ctx->shard_blob.p, cudaMemcpyDeviceToDevice, s);
+            // zero padding: the blob's bytes are those of the host partial, whatever the pool's memory held
+            if (L.probe > L.words * 4) CUDA_CHECK(cudaMemsetAsync(ctx->shard_blob.p + L.words * 4, 0, L.probe - L.words * 4, s));
+        });   // ms_search synchronises: the blob is complete when this call returns
+        if (rc) return rc;
+        meta[0] = A.p_begin; meta[1] = A.p_end; meta[2] = A.n_events; meta[3] = A.n_matches;
         *d_blob = ctx->shard_blob.p;
-        *blob_bytes = int64_t(total);
+        *blob_bytes = int64_t(L.bytes);
         return ASGART_B200_OK;
     });
 }
@@ -1774,48 +1794,7 @@ int32_t asgart_b200_ctx_finish_dev(asgart_b200_ctx* ctx, const asgart_b200_chunk
     return guarded(ctx, [&]() -> int32_t {
         if (!out || !d_blobs || !metas || n_shards < 1) return fail(ctx, ASGART_B200_EINVAL, "bad finish arguments");
         *out = nullptr;
-        if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "finish before load_strand");
-        ChunkPlan plan;
-        int rc = make_plan(ctx, chunks, n_chunks, st, plan);
-        if (rc) return rc;
-        u64 expect = 0, ne = 0, nm = 0;
-        for (int r = 0; r < n_shards; ++r) {
-            const u64 pb = metas[4 * r], pe = metas[4 * r + 1];
-            if (pb != expect || pe < pb || pe > plan.total_probes || ((pb & 31) && pb != plan.total_probes) || (!d_blobs[r] && pe > pb))
-                return fail(ctx, ASGART_B200_EINVAL, "partials are not the consecutive shards of this plan");
-            expect = pe;
-            ne += metas[4 * r + 2]; nm += metas[4 * r + 3];
-        }
-        if (expect != plan.total_probes) return fail(ctx, ASGART_B200_EINVAL, "partials do not cover all probes");
-        cudaStream_t s = ctx->stream;
-        const u64 words = ceil_div(plan.total_probes, 32);
-        DevBuf<u32> d_bits(words, s), d_cnt(ne, s);
-        DevBuf<u64> d_probe(ne, s), d_moff(ne, s), d_matches(nm, s);
-        u64 e0 = 0, m0 = 0;
-        for (int r = 0; r < n_shards; ++r) {
-            const u64 pb = metas[4 * r], pe = metas[4 * r + 1], re = metas[4 * r + 2], rm = metas[4 * r + 3];
-            const u64 w = ceil_div(pe - pb, 32), wbytes = ceil_div(w * 4, 8) * 8;
-            const u8* p = static_cast<const u8*>(d_blobs[r]);
-            if (w) CUDA_CHECK(cudaMemcpyAsync(d_bits.p + (pb >> 5), p, w * 4, cudaMemcpyDeviceToDevice, s));
-            p += wbytes;
-            if (re) CUDA_CHECK(cudaMemcpyAsync(d_probe.p + e0, p, re * 8, cudaMemcpyDeviceToDevice, s));
-            p += re * 8;
-            if (rm) CUDA_CHECK(cudaMemcpyAsync(d_matches.p + m0, p, rm * 8, cudaMemcpyDeviceToDevice, s));
-            p += rm * 8;
-            if (re) CUDA_CHECK(cudaMemcpyAsync(d_cnt.p + e0, p, re * 4, cudaMemcpyDeviceToDevice, s));
-            e0 += re; m0 += rm;
-        }
-        if (ne) {
-            const u32* cp = d_cnt.p; u64* mp = d_moff.p;
-            device_scan<u64, SumOp>([cp] __device__(u64 e) { return u64(cp[e]); }, [mp] __device__(u64 e, u64 exc, u64) { mp[e] = exc; },
-                                    ne, (u64*)nullptr, s);
-        }
-        asgart_b200_result* r = new asgart_b200_result();
-        try {
-            run_stage_b(ctx, plan, st, d_bits.p, ne, d_probe.p, d_cnt.p, d_moff.p, d_matches.p, nm, post_mask, r);
-        } catch (...) { delete r; throw; }
-        *out = r;
-        return ASGART_B200_OK;
+        return merge_shards(ctx, chunks, n_chunks, st, d_blobs, metas, n_shards, post_mask, out);
     });
 }
 

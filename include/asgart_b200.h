@@ -195,7 +195,10 @@ ASGART_B200_API void asgart_b200_hits_free(asgart_b200_hits *h);
 
 /* Multi-GPU (one process per GPU; strand + index replicated; probes partitioned by position):
  *   every rank: ctx_search_shard(rank, world) -> partial; exchange the serialised partials (NCCL all-gather);
- *   any rank:   ctx_finish(partials[world]) -> families (identical on every rank and for every world size). */
+ *   any rank:   ctx_finish(partials[world]) -> families (identical on every rank and for every world size).
+ * A serialised partial is a 48-byte header {magic, p_begin, p_end, events, matches, blob bytes} followed, byte for byte,
+ * by the blob that search_shard_dev leaves in HBM for the same shard. The bytes are opaque: they are valid only between
+ * processes that run the same build of this library. */
 ASGART_B200_API int32_t asgart_b200_ctx_search_shard(asgart_b200_ctx *ctx, const asgart_b200_chunk *chunks,
                                                      int64_t n_chunks, const asgart_b200_settings *settings,
                                                      int32_t shard, int32_t n_shards, asgart_b200_partial **out);
