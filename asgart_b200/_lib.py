@@ -103,6 +103,7 @@ SYMBOLS = [
     "asgart_b200_run_result_to_json", "asgart_b200_run_result_error", "asgart_b200_run_result_free",
     "asgart_b200_ctx_locate", "asgart_b200_hits_n_patterns", "asgart_b200_hits_first", "asgart_b200_hits_count",
     "asgart_b200_hits_offsets", "asgart_b200_hits_positions", "asgart_b200_hits_free",
+    "asgart_b200_ctx_copy_strand", "asgart_b200_search_group", "asgart_b200_run_files_devices",
 ]
 
 _lib = None
@@ -133,6 +134,8 @@ def load() -> C.CDLL:
         "asgart_b200_ctx_build_index_trim": (i32, [vp, C.c_uint64, C.c_uint64]),
         "asgart_b200_effective_trim": (i32, [C.c_uint64, C.c_uint64, i64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "asgart_b200_build_index_group": (i32, [C.POINTER(vp), i32]),
+        "asgart_b200_search_group": (i32, [C.POINTER(vp), i32, vp, i64, PS, u32, C.POINTER(vp)]),
+        "asgart_b200_ctx_copy_strand": (i32, [vp, vp]),
         "asgart_b200_dist_unique_id": (i32, [vp, i64]),
         "asgart_b200_ctx_dist_init": (i32, [vp, i32, i32, vp, i64]),
         "asgart_b200_ctx_dist_shutdown": (i32, [vp]),
@@ -188,6 +191,8 @@ def load() -> C.CDLL:
         "asgart_b200_run_files_passes": (vp, [C.c_char_p, PS, i32, i32, C.POINTER(C.c_char_p)]),
         "asgart_b200_run_files_sliced": (vp, [C.c_char_p, PS, i32, i32, u32, C.c_uint64, i64, C.POINTER(C.c_char_p)]),
         "asgart_b200_run_files_sliced_ex": (vp, [C.c_char_p, PS, i32, i32, C.POINTER(SliceOptions), C.POINTER(C.c_char_p)]),
+        "asgart_b200_run_files_devices": (vp, [C.c_char_p, PS, i32, C.POINTER(i32), i32, C.POINTER(SliceOptions),
+                                               C.POINTER(C.c_char_p)]),
         "asgart_b200_run_result_new": (vp, [vp, PS, vp, i64, vp]),
         "asgart_b200_run_result_slice": (i32, [vp, C.POINTER(SliceOptions)]),
         "asgart_b200_run_result_to_json": (vp, [vp]),

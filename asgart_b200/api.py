@@ -215,6 +215,24 @@ def build_index_group(ctxs: Sequence["Context"]):
         raise AsgartB200Error(rc, "; ".join(m for m in msgs if m))
 
 
+def search_group(ctxs: Sequence["Context"], chunks: Sequence[Tuple[int, int]], settings: RunSettings,
+                 post_mask: int = POST_ALL) -> Families:
+    """Search by several contexts of this process, each on its share of the probes (host threads); the first merges the
+    shares and applies the post-steps. Every context needs an index over the same strand (build_index_group, or one
+    build_index each). Gives the families of ``ctxs[0].search`` alone."""
+    L = _lib.load()
+    arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
+    ch = _chunks_array(chunks)
+    st = settings.to_c()
+    rh = C.c_void_p()
+    rc = L.asgart_b200_search_group(arr, len(ctxs), _ptr(ch), len(ch), C.byref(st), _with_score(settings, post_mask), C.byref(rh))
+    if rc != 0:
+        msgs = [f"member {r}: {L.asgart_b200_ctx_last_error(c.h).decode()}" for r, c in enumerate(ctxs)
+                if L.asgart_b200_ctx_last_error(c.h)]
+        raise AsgartB200Error(rc, "; ".join(msgs))
+    return _take_result(L, rh)
+
+
 class Context:
     """One device context: strand + index resident in HBM, searches run against it."""
 
@@ -281,6 +299,12 @@ class Context:
         out = np.empty(self.n1, dtype=np.uint8)
         self._check(self.L.asgart_b200_ctx_download_strand(self.h, _ptr(out), len(out)))
         return out
+
+    def copy_strand_from(self, other: "Context"):
+        """Take ``other``'s strand by a device-to-device copy (same or peer device); this context ends as after
+        load_strand: no index."""
+        self._check(self.L.asgart_b200_ctx_copy_strand(self.h, other.h))
+        self.n1 = other.n1
 
     def set_index_bits(self, bits: int):
         self._check(self.L.asgart_b200_ctx_set_index_bits(self.h, bits))
@@ -608,12 +632,23 @@ def out_filename(files: Sequence[str], settings: RunSettings, prefix: str = "", 
         L.asgart_b200_free_string(p)
 
 
-def search_duplications(files: Sequence[str], settings: RunSettings, device: int = 0) -> str:
-    """The whole `asgart FILES...` run (src/bin/asgart.rs:731-822) -> JSON text as JSONExporter::save writes it."""
+def _run_files_devices(L, files: Sequence[str], arr, n_passes: int, devices: Sequence[int], err):
+    dev = (C.c_int32 * len(devices))(*[int(d) for d in devices])
+    return L.asgart_b200_run_files_devices("\n".join(files).encode(), arr, n_passes, dev, len(devices), None, C.byref(err))
+
+
+def search_duplications(files: Sequence[str], settings: RunSettings, device: int = 0,
+                        devices: Optional[Sequence[int]] = None) -> str:
+    """The whole `asgart FILES...` run (src/bin/asgart.rs:731-822) -> JSON text as JSONExporter::save writes it.
+    ``devices``, when given, replaces ``device``: the run is shared by one context per entry (an entry may repeat) and
+    gives the same JSON as on one device."""
     L = _lib.load()
     st = settings.to_c()
     err = C.c_char_p()
-    p = L.asgart_b200_run_files("\n".join(files).encode(), C.byref(st), device, C.byref(err))
+    if devices is not None:
+        p = _run_files_devices(L, files, C.byref(st), 1, devices, err)
+    else:
+        p = L.asgart_b200_run_files("\n".join(files).encode(), C.byref(st), device, C.byref(err))
     if not p:
         raise AsgartB200Error(-1, err.value.decode() if err.value else "run failed")
     try:
@@ -622,13 +657,18 @@ def search_duplications(files: Sequence[str], settings: RunSettings, device: int
         L.asgart_b200_free_string(p)
 
 
-def search_duplications_passes(files: Sequence[str], passes: Sequence[RunSettings], device: int = 0) -> str:
+def search_duplications_passes(files: Sequence[str], passes: Sequence[RunSettings], device: int = 0,
+                               devices: Optional[Sequence[int]] = None) -> str:
     """Several runs (e.g. direct and -RC) over one index, combined as `asgart-slice` combines their JSON files
-    (RunResult::from_files, src/structs.rs:114-141): strand and settings of the first pass, families concatenated."""
+    (RunResult::from_files, src/structs.rs:114-141): strand and settings of the first pass, families concatenated.
+    ``devices`` as for search_duplications."""
     L = _lib.load()
     arr = (_lib.Settings * len(passes))(*[p.to_c() for p in passes])
     err = C.c_char_p()
-    p = L.asgart_b200_run_files_passes("\n".join(files).encode(), arr, len(passes), device, C.byref(err))
+    if devices is not None:
+        p = _run_files_devices(L, files, arr, len(passes), devices, err)
+    else:
+        p = L.asgart_b200_run_files_passes("\n".join(files).encode(), arr, len(passes), device, C.byref(err))
     if not p:
         raise AsgartB200Error(-1, err.value.decode() if err.value else "run failed")
     try:

@@ -1036,6 +1036,25 @@ int merge_shards(asgart_b200_ctx* ctx, const asgart_b200_chunk* chunks, i64 n_ch
     return ASGART_B200_OK;
 }
 
+// Peer access between the devices of `ctxs` (every ordered pair of distinct devices), for the members of a group and for
+// copy_strand: each reads the others' device memory. Failures are reported in `report`.
+int32_t enable_peer_access(const asgart_b200_ctx* const* ctxs, int n, asgart_b200_ctx* report) {
+    for (int a = 0; a < n; ++a)
+        for (int b = 0; b < n; ++b) {
+            if (ctxs[a]->device == ctxs[b]->device) continue;
+            int can = 0;
+            if (cudaDeviceCanAccessPeer(&can, ctxs[a]->device, ctxs[b]->device) != cudaSuccess || !can) {
+                cudaGetLastError();
+                return fail(report, ASGART_B200_EINVAL, "no peer access between the devices of the group");
+            }
+            cudaSetDevice(ctxs[a]->device);
+            cudaError_t e = cudaDeviceEnablePeerAccess(ctxs[b]->device, 0);
+            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return fail(report, ASGART_B200_ECUDA, cudaGetErrorString(e));
+            cudaGetLastError();
+        }
+    return ASGART_B200_OK;
+}
+
 void fold_family_timers(asgart_b200_ctx* ctx) {
     ctx->t_sort.drain(); ctx->t_gather.drain(); ctx->t_rank.drain(); ctx->t_probe.drain(); ctx->t_emit.drain(); ctx->t_scatter.drain(); ctx->t_scatter_main.drain();
     ctx->t_msd0.drain(); ctx->t_msd_hist.drain(); ctx->t_msd_local.drain();
@@ -1461,6 +1480,26 @@ int32_t asgart_b200_ctx_download_strand(asgart_b200_ctx* ctx, uint8_t* out, int6
     });
 }
 
+int32_t asgart_b200_ctx_copy_strand(asgart_b200_ctx* dst, const asgart_b200_ctx* src) {
+    if (!dst) return ASGART_B200_EINVAL;
+    if (!src || src == dst) return fail(dst, ASGART_B200_EINVAL, "copy_strand needs another context as its source");
+    return guarded(dst, [&]() -> int32_t {
+        if (!src->have_strand) return fail(dst, ASGART_B200_ESTATE, "copy_strand from a context without a strand");
+        const asgart_b200_ctx* pair[2] = {dst, src};
+        const int32_t prc = enable_peer_access(pair, 2, dst);
+        if (prc) return prc;
+        CUDA_CHECK(cudaSetDevice(dst->device));
+        dst->have_strand = dst->have_index = false;
+        drop_sorted_keys(dst);
+        dst->pn_mode = -1;
+        dst->n1 = src->n1;
+        // src's strand is complete: its load or ingest synchronised its stream before it set have_strand
+        dst->d_text.alloc(dst->n1, dst->stream);
+        CUDA_CHECK(cudaMemcpyAsync(dst->d_text.p, src->d_text.p, dst->n1, cudaMemcpyDefault, dst->stream));
+        return pack_loaded_strand(dst);
+    });
+}
+
 int32_t asgart_b200_ctx_build_index(asgart_b200_ctx* ctx) {
     return guarded(ctx, [&]() -> int32_t {
         if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "build_index before load_strand");
@@ -1515,17 +1554,8 @@ int32_t asgart_b200_build_index_group(asgart_b200_ctx* const* ctxs, int32_t worl
         if (!ctxs[r]->have_strand || ctxs[r]->n1 != ctxs[0]->n1) return fail(ctxs[r], ASGART_B200_ESTATE, "every member needs the same strand loaded");
     }
     // members on different devices reach each other's rank slices through peer access
-    for (int a = 0; a < world; ++a)
-        for (int b2 = 0; b2 < world; ++b2) {
-            if (ctxs[a]->device == ctxs[b2]->device) continue;
-            int can = 0;
-            if (cudaDeviceCanAccessPeer(&can, ctxs[a]->device, ctxs[b2]->device) != cudaSuccess || !can)
-                return fail(ctxs[a], ASGART_B200_EINVAL, "no peer access between the devices of the group");
-            cudaSetDevice(ctxs[a]->device);
-            cudaError_t e = cudaDeviceEnablePeerAccess(ctxs[b2]->device, 0);
-            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return fail(ctxs[a], ASGART_B200_ECUDA, cudaGetErrorString(e));
-            cudaGetLastError();
-        }
+    const int32_t prc = enable_peer_access(ctxs, world, ctxs[0]);
+    if (prc) return prc;
     ThreadGroupShared shared(world);
     std::vector<int32_t> rc(world, ASGART_B200_OK);
     std::vector<std::thread> threads;
@@ -1542,6 +1572,55 @@ int32_t asgart_b200_build_index_group(asgart_b200_ctx* const* ctxs, int32_t worl
     for (int r = 0; r < world; ++r)
         if (rc[r] != ASGART_B200_OK) return rc[r];
     return ASGART_B200_OK;
+}
+
+// Search counterpart of build_index_group: member r runs stage A over probe shard r of `world` on its own host thread and
+// leaves its partial in its HBM (search_shard_dev); member 0 merges the partials (merge_shards) and runs stage B. A blob on
+// member 0's device is read where it lies; a blob on another device is first copied into one buffer on member 0's device,
+// on member 0's stream, once that member's stage A has returned (its stream is then idle).
+int32_t asgart_b200_search_group(asgart_b200_ctx* const* ctxs, int32_t world, const asgart_b200_chunk* chunks, int64_t n_chunks,
+                                 const asgart_b200_settings* st, uint32_t post_mask, asgart_b200_result** out) {
+    if (!ctxs || world < 1 || world > kMaxWorld || !out) return ASGART_B200_EINVAL;
+    *out = nullptr;
+    for (int r = 0; r < world; ++r) {
+        if (!ctxs[r]) return ASGART_B200_EINVAL;
+        for (int q = 0; q < r; ++q)
+            if (ctxs[q] == ctxs[r]) return fail(ctxs[r], ASGART_B200_EINVAL, "a context is a member of the group twice");
+    }
+    for (int r = 0; r < world; ++r) ctxs[r]->err.clear();   // afterwards, the members that failed say why
+    for (int r = 0; r < world; ++r)
+        if (!ctxs[r]->have_index || ctxs[r]->n1 != ctxs[0]->n1 || ctxs[r]->sa_len != ctxs[0]->sa_len)
+            return fail(ctxs[r], ASGART_B200_ESTATE, "every member needs an index over the same strand");
+    const int32_t prc = enable_peer_access(ctxs, world, ctxs[0]);
+    if (prc) return prc;
+    std::vector<int32_t> rc(world, ASGART_B200_OK);
+    std::vector<void*> blobs(world, nullptr);
+    std::vector<int64_t> bytes(world, 0);
+    std::vector<u64> metas(4 * size_t(world), 0);
+    std::vector<std::thread> threads;
+    for (int r = 0; r < world; ++r)
+        threads.emplace_back([&, r] {
+            rc[r] = asgart_b200_ctx_search_shard_dev(ctxs[r], chunks, n_chunks, st, r, world, &blobs[r], &bytes[r], &metas[4 * size_t(r)]);
+        });
+    for (auto& t : threads) t.join();
+    for (int r = 0; r < world; ++r)
+        if (rc[r] != ASGART_B200_OK) return rc[r];
+    asgart_b200_ctx* c0 = ctxs[0];
+    return guarded(c0, [&]() -> int32_t {
+        u64 far = 0;
+        for (int r = 1; r < world; ++r)
+            if (ctxs[r]->device != c0->device) far += u64(bytes[r]);
+        DevBuf<u8> gathered(far, c0->stream);
+        std::vector<const void*> d_blobs(blobs.begin(), blobs.end());
+        u64 at = 0;
+        for (int r = 1; r < world; ++r) {
+            if (ctxs[r]->device == c0->device || bytes[r] == 0) continue;
+            CUDA_CHECK(cudaMemcpyAsync(gathered.p + at, blobs[r], size_t(bytes[r]), cudaMemcpyDefault, c0->stream));
+            d_blobs[r] = gathered.p + at;
+            at += u64(bytes[r]);
+        }
+        return merge_shards(c0, chunks, n_chunks, st, d_blobs.data(), metas.data(), world, post_mask, out);
+    });
 }
 
 int32_t asgart_b200_dist_unique_id(uint8_t* out, int64_t cap) {

@@ -3,6 +3,7 @@
 // (naming rule src/bin/asgart.rs:695-719).
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -29,6 +30,7 @@ static void usage() {
             "      --keep-fragments <A,B,..> --restrict-fragments <A,B,..> --exclude-fragments <A,B,..> [--regexp]\n"
             "                              asgart-slice's fragment options (they rewrite the fragment map)\n"
             "      --device <N>            CUDA device [default: 0]\n"
+            "      --devices <A,B,..>      run on several CUDA devices at once (a device may repeat); not with --device or --trim\n"
             "      --with-direct           (with -R/-C) also run the direct pass on the same index and write both, combined as\n"
             "                              `asgart-slice` combines the two runs' files\n"
             "      --threads, --chunk-size accepted and ignored (the reference ignores --chunk-size too)\n"
@@ -42,6 +44,8 @@ int main(int argc, char** argv) {
     std::string prefix, out;
     std::vector<std::string> files;
     int device = 0, verbose = 0, with_direct = 0;
+    bool have_device = false;
+    std::vector<int32_t> devices;
     uint32_t slice_flags = 0;
     uint64_t slice_min = 0;
     long long slice_max = -1;
@@ -58,7 +62,20 @@ int main(int argc, char** argv) {
         else if (a == "--max-cardinality") st.max_cardinality = strtoull(need(i), nullptr, 10);
         else if (a == "--prefix") prefix = need(i);
         else if (a == "--out") out = need(i);
-        else if (a == "--device") device = atoi(need(i));
+        else if (a == "--device") { device = atoi(need(i)); have_device = true; }
+        else if (a == "--devices") {
+            devices.clear();
+            const std::string v = need(i);
+            for (size_t b = 0; b <= v.size();) {
+                const size_t e = std::min(v.find(',', b), v.size());
+                const std::string d = v.substr(b, e - b);
+                char* end = nullptr;
+                const long n = strtol(d.c_str(), &end, 10);
+                if (d.empty() || *end || n < 0) { usage(); return 2; }
+                devices.push_back(int32_t(n));
+                b = e + 1;
+            }
+        }
         else if (a == "--threads" || a == "--chunk-size") need(i);
         else if (a == "--compute-score") st.compute_score = 1;
         else if (a == "--with-direct") with_direct = 1;
@@ -90,7 +107,8 @@ int main(int argc, char** argv) {
         else if (a[0] == '-') { usage(); return 2; }
         else files.push_back(a);
     }
-    if (files.empty()) { usage(); return 2; }
+    if (files.empty() || (have_device && !devices.empty())) { usage(); return 2; }
+    if (devices.empty()) devices.push_back(device);
     st.max_gap_size = uint32_t(gap + st.probe_size);  // src/bin/asgart.rs:681
     std::string joined;
     for (size_t i = 0; i < files.size(); ++i) joined += (i ? "\n" : "") + files[i];
@@ -103,8 +121,8 @@ int main(int argc, char** argv) {
     op.keep_fragments = have_keep ? keep_f.c_str() : nullptr;
     op.restrict_fragments = have_restrict ? restrict_f.c_str() : nullptr;
     op.exclude_fragments = have_exclude ? exclude_f.c_str() : nullptr;
-    char* js = slice ? asgart_b200_run_files_sliced_ex(joined.c_str(), passes, n_passes, device, &op, &err)
-                     : asgart_b200_run_files_passes(joined.c_str(), passes, n_passes, device, &err);
+    char* js = asgart_b200_run_files_devices(joined.c_str(), passes, n_passes, devices.data(), int32_t(devices.size()),
+                                             slice ? &op : nullptr, &err);
     if (!js) { fprintf(stderr, "asgart-b200: %s\n", err ? err : "failed"); return 1; }
     char* name = asgart_b200_out_filename(joined.c_str(), prefix.c_str(), out.empty() ? nullptr : out.c_str(), &st);
     FILE* f = fopen(name, "wb");

@@ -837,46 +837,66 @@ char* asgart_b200_out_filename(const char* files, const char* prefix, const char
 // bin/asgart.rs:731-822: prepare_data -> SearchDuplications -> FilterNs -> ReOrder -> ReduceOverlap -> Sort -> JSON,
 // for one or several passes over ONE index. prepare_data runs on the device too (GPU-side FASTA ingest): the files'
 // bytes go to HBM as they are read. Several passes combine as RunResult::from_files does for their JSON files
-// (structs.rs:114-141): strand and settings of the first, families concatenated in pass order.
-static char* run_files_impl(const char* files, const asgart_b200_settings* passes, int32_t n_passes, int32_t device,
-                            const asgart_b200_slice_options* slice, const char** err) {
+// (structs.rs:114-141): strand and settings of the first, families concatenated in pass order. With several devices,
+// member 0 ingests, the others copy its strand, and the group builds the index and searches every pass.
+static char* run_files_impl(const char* files, const asgart_b200_settings* passes, int32_t n_passes, const int32_t* devices,
+                            int32_t n_devices, const asgart_b200_slice_options* slice, const char** err) {
     static thread_local std::string msg;
     if (err) *err = nullptr;
     auto failf = [&](const std::string& m) -> char* { msg = m; if (err) *err = msg.c_str(); return nullptr; };
     if (!passes || n_passes < 1) return failf("no passes");
+    if (!devices || n_devices < 1) return failf("no devices");
     for (int32_t i = 1; i < n_passes; ++i)
         if ((passes[i].skip_masked != 0) != (passes[0].skip_masked != 0))
             return failf("passes over one index must agree on skip_masked (it changes the strand)");
     for (int32_t i = 1; i < n_passes; ++i)
         if (passes[i].has_trim != passes[0].has_trim || passes[i].trim_a != passes[0].trim_a || passes[i].trim_b != passes[0].trim_b)
             return failf("passes over one index must agree on trim (it changes the index)");
+    if (passes[0].has_trim && n_devices > 1) return failf("--trim builds its index on one device: give one device, not " + std::to_string(n_devices));
     const std::vector<std::string> fl = split_lines(files);
     if (fl.empty()) return failf("no input files");
-    asgart_b200_ctx* ctx = nullptr;
-    int rc = asgart_b200_ctx_create(device, &ctx);
-    if (rc) return failf("no usable CUDA device (code " + std::to_string(rc) + "); this build has no CPU path");
+    std::vector<asgart_b200_ctx*> ctxs(size_t(n_devices), nullptr);
+    int rc = 0;
+    for (int32_t i = 0; !rc && i < n_devices; ++i) {
+        rc = asgart_b200_ctx_create(devices[i], &ctxs[size_t(i)]);
+        if (rc && n_devices == 1) failf("no usable CUDA device (code " + std::to_string(rc) + "); this build has no CPU path");
+        else if (rc) failf("cannot use CUDA device " + std::to_string(devices[i]) + " (code " + std::to_string(rc) + "); this build has no CPU path");
+    }
+    asgart_b200_ctx* ctx = ctxs[0];
+    auto last_error = [&]() -> std::string {   // the first member that says why it failed
+        for (asgart_b200_ctx* c : ctxs)
+            if (c && *asgart_b200_ctx_last_error(c)) return asgart_b200_ctx_last_error(c);
+        return "code " + std::to_string(rc);
+    };
     asgart_b200_prepared* p = nullptr;
     char* js = nullptr;
-    rc = asgart_b200_ctx_ingest_begin(ctx);
-    for (size_t i = 0; !rc && i < fl.size(); ++i) rc = asgart_b200_ctx_ingest_file(ctx, fl[i].c_str(), int32_t(passes[0].skip_masked));
-    if (!rc) rc = asgart_b200_ctx_ingest_finish(ctx, files, &p);
-    if (rc) {
-        failf(asgart_b200_ctx_last_error(ctx));
-    } else {
+    if (!rc) {
+        rc = asgart_b200_ctx_ingest_begin(ctx);
+        for (size_t i = 0; !rc && i < fl.size(); ++i) rc = asgart_b200_ctx_ingest_file(ctx, fl[i].c_str(), int32_t(passes[0].skip_masked));
+        if (!rc) rc = asgart_b200_ctx_ingest_finish(ctx, files, &p);
+        if (rc) failf(asgart_b200_ctx_last_error(ctx));
+    }
+    if (!rc) {
         std::vector<uint64_t> fam_off{0};
         std::vector<asgart_b200_protosd> sds;
         // --trim (bin/asgart.rs:432-463 validation, :142-147 index); the raw values stay in the settings block of the JSON
         uint64_t ta = 0, tb = 0;
         int64_t n_plus_1 = 0;
         asgart_b200_prepared_strand(p, &n_plus_1);
-        if (passes[0].has_trim && asgart_b200_effective_trim(passes[0].trim_a, passes[0].trim_b, n_plus_1, &ta, &tb))
+        if (n_devices > 1) {
+            for (int32_t i = 1; !rc && i < n_devices; ++i) rc = asgart_b200_ctx_copy_strand(ctxs[size_t(i)], ctx);
+            if (!rc) rc = asgart_b200_build_index_group(ctxs.data(), n_devices);
+        } else if (passes[0].has_trim && asgart_b200_effective_trim(passes[0].trim_a, passes[0].trim_b, n_plus_1, &ta, &tb)) {
             rc = asgart_b200_ctx_build_index_trim(ctx, ta, tb);
-        else
+        } else {
             rc = asgart_b200_ctx_build_index(ctx);
+        }
         for (int32_t i = 0; !rc && i < n_passes; ++i) {
             asgart_b200_result* res = nullptr;
-            rc = asgart_b200_ctx_search(ctx, p->chunks.data(), int64_t(p->chunks.size()), &passes[i],
-                                        ASGART_B200_POST_ALL | (passes[i].compute_score ? ASGART_B200_POST_COMPUTE_SCORE : 0u), &res);
+            const uint32_t post = ASGART_B200_POST_ALL | (passes[i].compute_score ? ASGART_B200_POST_COMPUTE_SCORE : 0u);
+            const int64_t nc = int64_t(p->chunks.size());
+            rc = n_devices > 1 ? asgart_b200_search_group(ctxs.data(), n_devices, p->chunks.data(), nc, &passes[i], post, &res)
+                               : asgart_b200_ctx_search(ctx, p->chunks.data(), nc, &passes[i], post, &res);
             if (!rc) {
                 const int64_t nf = asgart_b200_result_n_families(res);
                 const uint64_t* off = asgart_b200_result_family_offsets(res);
@@ -886,7 +906,7 @@ static char* run_files_impl(const char* files, const asgart_b200_settings* passe
             }
             asgart_b200_result_free(res);
         }
-        if (rc) failf(std::string("device pipeline failed: ") + asgart_b200_ctx_last_error(ctx));
+        if (rc) failf("device pipeline failed: " + last_error());
         else if (!slice) js = asgart_b200_to_json(p, &passes[0], fam_off.data(), int64_t(fam_off.size()) - 1, sds.data());
         else {
             asgart_b200_run_result* rr = asgart_b200_run_result_new(p, &passes[0], fam_off.data(), int64_t(fam_off.size()) - 1, sds.data());
@@ -896,26 +916,31 @@ static char* run_files_impl(const char* files, const asgart_b200_settings* passe
             asgart_b200_run_result_free(rr);
         }
     }
-    asgart_b200_ctx_destroy(ctx);
+    for (asgart_b200_ctx* c : ctxs) asgart_b200_ctx_destroy(c);
     if (p) asgart_b200_prepared_free(p);
     return js;
 }
 
 char* asgart_b200_run_files_passes(const char* files, const asgart_b200_settings* passes, int32_t n_passes, int32_t device,
                                    const char** err) {
-    return run_files_impl(files, passes, n_passes, device, nullptr, err);
+    return run_files_impl(files, passes, n_passes, &device, 1, nullptr, err);
 }
 
 char* asgart_b200_run_files_sliced(const char* files, const asgart_b200_settings* passes, int32_t n_passes, int32_t device,
                                    uint32_t slice_flags, uint64_t min_length, int64_t max_family_members, const char** err) {
     asgart_b200_slice_options op{};
     op.flags = slice_flags; op.min_length = min_length; op.max_family_members = max_family_members;
-    return run_files_impl(files, passes, n_passes, device, &op, err);
+    return run_files_impl(files, passes, n_passes, &device, 1, &op, err);
 }
 
 char* asgart_b200_run_files_sliced_ex(const char* files, const asgart_b200_settings* passes, int32_t n_passes, int32_t device,
                                       const asgart_b200_slice_options* options, const char** err) {
-    return run_files_impl(files, passes, n_passes, device, options, err);
+    return run_files_impl(files, passes, n_passes, &device, 1, options, err);
+}
+
+char* asgart_b200_run_files_devices(const char* files, const asgart_b200_settings* passes, int32_t n_passes, const int32_t* devices,
+                                    int32_t n_devices, const asgart_b200_slice_options* options, const char** err) {
+    return run_files_impl(files, passes, n_passes, devices, n_devices, options, err);
 }
 
 char* asgart_b200_run_files(const char* files, const asgart_b200_settings* st, int32_t device, const char** err) {

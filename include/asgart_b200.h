@@ -131,12 +131,21 @@ ASGART_B200_API int32_t asgart_b200_effective_trim(uint64_t start, uint64_t stop
  * in each other's memory (peer stores / loads over NVLink) and end with the whole index on every member, bit-identical
  * to a single-device build. Every member must have the same strand loaded.
  *   one process, several contexts (any devices with peer access, or all on one device): build_index_group runs the
- *     members on host threads;
+ *     members on host threads, and search_group (below) searches with them;
  *   one process per GPU: rank 0 makes a unique id (dist_unique_id, 128 bytes) and sends it to the others by any means
  *     (asgart_b200/dist.py: torch.distributed broadcast); every rank calls ctx_dist_init, after which ctx_build_index is
  *     a collective call (NCCL for the phase boundaries and the final exchange of SA pieces, CUDA IPC for the peer
  *     pointers) until ctx_dist_shutdown. */
 ASGART_B200_API int32_t asgart_b200_build_index_group(asgart_b200_ctx *const *ctxs, int32_t world);
+/* Search counterpart of build_index_group for the contexts of one process: member r searches probe shard r of `world`
+ * (ctx_search_shard_dev) on its own host thread, member 0 merges the shards' partials (ctx_finish_dev) and applies the
+ * post-steps of post_mask. The families equal those of ctx_search on member 0 alone, for every world. Every member needs
+ * an index over the same strand (same n + 1, same index length): ASGART_B200_ESTATE otherwise. On failure the call
+ * returns the first failing member's code and that member's last_error says why (every member's last_error is cleared
+ * when the call starts); all members stay usable. */
+ASGART_B200_API int32_t asgart_b200_search_group(asgart_b200_ctx *const *ctxs, int32_t world, const asgart_b200_chunk *chunks,
+                                                 int64_t n_chunks, const asgart_b200_settings *settings, uint32_t post_mask,
+                                                 asgart_b200_result **out);
 ASGART_B200_API int32_t asgart_b200_dist_unique_id(uint8_t *out, int64_t cap);   /* returns the id size (128) */
 ASGART_B200_API int32_t asgart_b200_ctx_dist_init(asgart_b200_ctx *ctx, int32_t rank, int32_t world,
                                                   const uint8_t *unique_id, int64_t id_bytes);
@@ -378,6 +387,14 @@ ASGART_B200_API void asgart_b200_run_result_free(asgart_b200_run_result *rr);
 /* asgart_b200_run_files_passes followed by asgart_b200_run_result_slice before the JSON is written */
 ASGART_B200_API char *asgart_b200_run_files_sliced_ex(const char *files, const asgart_b200_settings *passes, int32_t n_passes,
                                                       int32_t device, const asgart_b200_slice_options *options, const char **err);
+/* asgart_b200_run_files_sliced_ex on several devices (options NULL: no slicing). One context per entry of devices (an
+ * entry may repeat: several members on one GPU); member 0 ingests the files, the others copy its strand
+ * (ctx_copy_strand), build_index_group builds the index and search_group runs every pass. The JSON is byte for byte the
+ * one-device run's. n_devices == 1 is the one-device path itself. --trim (has_trim) builds on one device only and is
+ * refused with more than one. */
+ASGART_B200_API char *asgart_b200_run_files_devices(const char *files, const asgart_b200_settings *passes, int32_t n_passes,
+                                                    const int32_t *devices, int32_t n_devices,
+                                                    const asgart_b200_slice_options *options, const char **err);
 
 /* ---- GPU-side FASTA ingest (SURVEY §8f row N1) ----------------------------------------------------------------
  * read_fasta + find_chunks_to_process of prepare_data (src/bin/asgart.rs:278-366) on the device, for the raw bytes of
@@ -400,6 +417,10 @@ ASGART_B200_API int32_t asgart_b200_ctx_ingest_finish(asgart_b200_ctx *ctx, cons
                                                       asgart_b200_prepared **out);
 /* the strand held by the context (n+1 bytes incl. '$') back to host memory; cap >= n+1 */
 ASGART_B200_API int32_t asgart_b200_ctx_download_strand(asgart_b200_ctx *ctx, uint8_t *out, int64_t cap);
+/* dst gets src's strand by a device-to-device copy (same device, or a peer device: peer access is enabled) and ends as
+ * ctx_load_strand leaves a context: packed, no index. How the members of a group get the strand that member 0 ingested,
+ * without reading the files again. ASGART_B200_ESTATE when src holds no strand. */
+ASGART_B200_API int32_t asgart_b200_ctx_copy_strand(asgart_b200_ctx *dst, const asgart_b200_ctx *src);
 
 /* ---- deterministic synthetic genomes (bench/test input; DESIGN.md "Synthetic inputs") ---------------------- */
 /* Fills out[0..n) (no '$') with the config's sequence (upper/lower case ACGT and N). config: 1..5 = BASELINE.json
