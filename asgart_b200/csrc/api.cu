@@ -6,6 +6,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <variant>
 #include <vector>
 
 #include <fcntl.h>
@@ -30,8 +31,12 @@ thread_local DevicePool* g_device_pool = nullptr;
 // keys: the build's sorted initial keys (keys[i] = first key_p0 symbols of suffix SA[i], key_b bits each, first symbol on
 // top), kept for the probe search when build_index ran on one device with lazy ranks; key_map = strand code (CODE_*) ->
 // key code, one nibble each (0xF: the symbol does not occur in the strand)
-struct Index32 { DevBuf<u32> sa, lut_lo, lut_hi, deep; int deep_depth = 0; DevBuf<u64> keys; int key_b = 0, key_p0 = 0; u64 key_map = 0; };
-struct Index64 { DevBuf<u64> sa, lut_lo, lut_hi, deep; int deep_depth = 0; DevBuf<u64> keys; int key_b = 0, key_p0 = 0; u64 key_map = 0; };
+template <typename IdxT>
+struct Index { DevBuf<IdxT> sa, lut_lo, lut_hi, deep; int deep_depth = 0; DevBuf<u64> keys; int key_b = 0, key_p0 = 0; u64 key_map = 0; };
+
+// kernel families timed on the context's stream, one FamilyTimer each (fold_family_timers maps them onto the stats)
+enum Family { FAM_SORT, FAM_GATHER, FAM_RANK, FAM_PROBE, FAM_EMIT, FAM_SCATTER, FAM_SCATTER_MAIN, FAM_MSD0, FAM_MSD_HIST, FAM_MSD_LOCAL,
+              FAM_LOCATE, FAM_COUNT };
 
 struct ChunkPlan {
     std::vector<ChunkDev> host;
@@ -66,15 +71,14 @@ struct asgart_b200_ctx {
     u64 n1 = 0;
     u64 sa_len = 0;    // entries of the suffix array: n1, or b - a + 1 for an index built with --trim (a, b)
     bool have_strand = false, have_index = false;
-    int want_bits = 0, idx_bits = 0;
+    int want_bits = 0;
     DevBuf<u8> d_text;
     DevBuf<u64> d_pt, d_pn;
     DevBuf<u8> shard_blob;   // device-resident partial of the last search_shard_dev call
     int pn_mode = -1;
-    Index32 ix32;
-    Index64 ix64;
+    std::variant<std::monostate, Index<u32>, Index<u64>> ix;   // the index of the last install (monostate: none yet)
     asgart_b200_stats st{};
-    FamilyTimer t_sort, t_gather, t_rank, t_probe, t_emit, t_scatter, t_scatter_main, t_msd0, t_msd_hist, t_msd_local;
+    FamilyTimer fam[FAM_COUNT];
     cudaEvent_t ev_a = nullptr, ev_b = nullptr;
     LaunchCounter launches;
     // sharded index build: the group this context is a member of (null: builds alone) and this member's slice of the
@@ -89,10 +93,8 @@ struct asgart_b200_ctx {
     std::vector<IngestPiece> pieces;
     u8* stage[2] = {nullptr, nullptr};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
-    // ctx_locate: its kernels' device time, pinned staging of its copies
-    FamilyTimer t_locate;
     u64 n_probe_keys = 0;   // asgart_b200_ctx_probe_keys
-    u8* loc_stage = nullptr;
+    u8* loc_stage = nullptr;   // ctx_locate: pinned staging of its copies
 };
 
 struct asgart_b200_hits {
@@ -204,30 +206,59 @@ void ingest_record_ids(IngestPiece& piece, u64 n, Fetch fetch) {
     }
 }
 
-template <typename IdxT> struct IxOf;
-template <> struct IxOf<u32> { static Index32& get(asgart_b200_ctx* c) { return c->ix32; } };
-template <> struct IxOf<u64> { static Index64& get(asgart_b200_ctx* c) { return c->ix64; } };
+// Calls f(Index<u32>&) or f(Index<u64>&) with the index the context holds (the caller checked have_index). nvcc does not
+// allow an extended __device__ lambda inside a generic lambda, so f only forwards to named templates.
+template <typename F>
+decltype(auto) with_index(asgart_b200_ctx* ctx, F&& f) {
+    if (auto* ix = std::get_if<Index<u32>>(&ctx->ix)) return f(*ix);
+    return f(std::get<Index<u64>>(ctx->ix));
+}
 
 // the sorted keys describe the strand and the index they were built with: a new strand, a new index or another index
 // width makes them stale
-void drop_sorted_keys(asgart_b200_ctx* ctx) { ctx->ix32.keys.release(); ctx->ix64.keys.release(); }
+void drop_sorted_keys(asgart_b200_ctx* ctx) {
+    if (!std::holds_alternative<std::monostate>(ctx->ix)) with_index(ctx, [](auto& ix) { ix.keys.release(); });
+}
+
+// a new strand makes the index, its sorted keys and the needle image stale
+void forget_strand(asgart_b200_ctx* ctx) {
+    ctx->have_strand = ctx->have_index = false;
+    drop_sorted_keys(ctx);
+    ctx->pn_mode = -1;
+}
+
+// 32-bit indices need n+1 < 2^32-2
+bool fits_u32_index(u64 n1) { return n1 < 0xFFFFFFFEull; }
 
 int pick_bits(const asgart_b200_ctx* ctx) {
     if (ctx->want_bits == 32 || ctx->want_bits == 64) return ctx->want_bits;
-    return (ctx->n1 < 0xFFFFFFFEull) ? 32 : 64;
+    return fits_u32_index(ctx->n1) ? 32 : 64;
+}
+
+// The install of every index (build_index, build_index_trim, upload_sa), after the entry point's own checks: the width,
+// then a fresh Index of that width in place of the held one, then build(ix). The old index goes back to the block cache
+// before the builder allocates: the sort's key buffers take the old sorted keys' block again.
+template <typename F>
+int32_t install_index(asgart_b200_ctx* ctx, u64 sa_len, F build) {
+    ctx->have_index = false;
+    const int bits = pick_bits(ctx);
+    if (bits == 32 && !fits_u32_index(ctx->n1)) return fail(ctx, ASGART_B200_EINVAL, "32-bit indices need n+1 < 2^32-2");
+    if (bits == 32) ctx->ix.emplace<Index<u32>>();
+    else ctx->ix.emplace<Index<u64>>();
+    with_index(ctx, build);
+    CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+    ctx->sa_len = sa_len;
+    ctx->have_index = true;
+    return ASGART_B200_OK;
 }
 
 // LUT from the finished suffix array (used when the index is uploaded, or the initial keys were shorter than 8 symbols)
 template <typename IdxT>
-void build_lut(asgart_b200_ctx* ctx) {
-    auto& ix = IxOf<IdxT>::get(ctx);
+void build_lut(asgart_b200_ctx* ctx, Index<IdxT>& ix) {
     ix.lut_lo.alloc(kLutSize, ctx->stream);
     ix.lut_hi.alloc(kLutSize, ctx->stream);
     ix.lut_lo.zero();
     ix.lut_hi.zero();
-    ix.deep.release();
-    ix.deep_depth = 0;
-    ix.keys.release();
     lut_build_kernel<IdxT><<<unsigned(ceil_div(ctx->n1, 256)), 256, 0, ctx->stream>>>(ctx->d_pt.p, ix.sa.p, ctx->n1, ix.lut_lo.p,
                                                                                       ix.lut_hi.p);
     KERNEL_CHECK();
@@ -238,23 +269,22 @@ void build_lut(asgart_b200_ctx* ctx) {
 template <typename IdxT>
 struct LutHook : SaKeyHook {
     asgart_b200_ctx* ctx;
+    Index<IdxT>& ix;
     bool done = false;
     double ms = 0;
     u64 m4 = 0, m5 = 0;
-    explicit LutHook(asgart_b200_ctx* c) : ctx(c) {}
+    LutHook(asgart_b200_ctx* c, Index<IdxT>& i) : ctx(c), ix(i) {}
     bool lookup_tables(SaLookupTables& t) override {
         if (!done) return false;
-        auto& ix = IxOf<IdxT>::get(ctx);
         t.deep = ix.deep.p; t.depth = ix.deep_depth; t.lut_lo = ix.lut_lo.p; t.lut_hi = ix.lut_hi.p; t.m4 = m4; t.m5 = m5;
         return ix.deep.p != nullptr;
     }
     void adopt_sorted_keys(DevBuf<u64>& keys) override {
-        if (done) IxOf<IdxT>::get(ctx).keys = std::move(keys);
+        if (done) ix.keys = std::move(keys);
     }
     void on_sorted_keys(const u64* d_keys, u64 n_local, u64 base, u64 n, int b, int p0, const uint16_t* h_code, cudaStream_t stream,
                         SaGroup* grp) override {
         if (p0 < 8 || n != ctx->n1) return;
-        auto& ix = IxOf<IdxT>::get(ctx);
         EventTimer t(stream);
         t.start();
         LutCodeMap map;
@@ -376,18 +406,23 @@ struct LutHook : SaKeyHook {
     }
 };
 
+// the suffix-array build's kernel families, timed by the context's timers
+SaStats sa_stats(asgart_b200_ctx* ctx) {
+    FamilyTimer* f = ctx->fam;
+    SaStats ss;
+    ss.sort = &f[FAM_SORT]; ss.gather = &f[FAM_GATHER]; ss.rank = &f[FAM_RANK]; ss.scatter = &f[FAM_SCATTER]; ss.scatter_main = &f[FAM_SCATTER_MAIN];
+    ss.msd.scatter = &f[FAM_SCATTER_MAIN]; ss.msd.scatter0 = &f[FAM_MSD0]; ss.msd.hist = &f[FAM_MSD_HIST]; ss.msd.local = &f[FAM_MSD_LOCAL];
+    return ss;
+}
+
 template <typename IdxT>
-void build_index_t(asgart_b200_ctx* ctx) {
+void build_index_t(asgart_b200_ctx* ctx, Index<IdxT>& ix) {
     NvtxRange nv("build_index");
-    auto& ix = IxOf<IdxT>::get(ctx);
-    ix.keys.release();   // before the sort allocates its key buffers: they take this block again
     EventTimer tsa(ctx->stream), tlut(ctx->stream);
     tsa.start();
     ix.sa.alloc(ctx->n1, ctx->stream);
-    LutHook<IdxT> hook(ctx);
-    SaStats ss;
-    ss.sort = &ctx->t_sort; ss.gather = &ctx->t_gather; ss.rank = &ctx->t_rank; ss.scatter = &ctx->t_scatter; ss.scatter_main = &ctx->t_scatter_main;
-    ss.msd.scatter = &ctx->t_scatter_main; ss.msd.scatter0 = &ctx->t_msd0; ss.msd.hist = &ctx->t_msd_hist; ss.msd.local = &ctx->t_msd_local;
+    LutHook<IdxT> hook(ctx, ix);
+    SaStats ss = sa_stats(ctx);
     SaGroup* grp = (ctx->group && ctx->group->world > 1) ? ctx->group : nullptr;
     if (!grp) {
         DevBuf<IdxT> rank(ctx->n1, ctx->stream);
@@ -416,16 +451,14 @@ void build_index_t(asgart_b200_ctx* ctx) {
     ctx->st.msd_levels = ss.used_msd ? u64(ss.msd.levels) : 0;
     tsa.stop();
     tlut.start();
-    if (!hook.done) build_lut<IdxT>(ctx);
+    if (!hook.done) build_lut(ctx, ix);
     tlut.stop();
     ctx->st.ms_sa_build += tsa.ms() - hook.ms;
     ctx->st.ms_lut += tlut.ms() + hook.ms;
 }
 
 template <typename IdxT>
-void build_index_trim_t(asgart_b200_ctx* ctx, u64 a, u64 b) {
-    auto& ix = IxOf<IdxT>::get(ctx);
-    ix.keys.release();
+void build_index_trim_t(asgart_b200_ctx* ctx, Index<IdxT>& ix, u64 a, u64 b) {
     cudaStream_t s = ctx->stream;
     EventTimer tsa(s), tlut(s);
     tsa.start();
@@ -434,9 +467,7 @@ void build_index_trim_t(asgart_b200_ctx* ctx, u64 a, u64 b) {
     CUDA_CHECK(cudaMemcpyAsync(sub.p, ctx->d_text.p + a, b - a, cudaMemcpyDeviceToDevice, s));
     CUDA_CHECK(cudaMemsetAsync(sub.p + (b - a), '$', 1, s));
     ix.sa.alloc(m1, s);
-    SaStats ss;
-    ss.sort = &ctx->t_sort; ss.gather = &ctx->t_gather; ss.rank = &ctx->t_rank; ss.scatter = &ctx->t_scatter; ss.scatter_main = &ctx->t_scatter_main;
-    ss.msd.scatter = &ctx->t_scatter_main; ss.msd.scatter0 = &ctx->t_msd0; ss.msd.hist = &ctx->t_msd_hist; ss.msd.local = &ctx->t_msd_local;
+    SaStats ss = sa_stats(ctx);
     {
         DevBuf<IdxT> rank(m1, s);
         build_suffix_array<IdxT>(sub.p, m1, ix.sa.p, rank.p, s, &ss, nullptr);
@@ -451,8 +482,6 @@ void build_index_trim_t(asgart_b200_ctx* ctx, u64 a, u64 b) {
     tlut.start();
     ix.lut_lo.alloc(kLutSize, s);
     ix.lut_hi.alloc(kLutSize, s);
-    ix.deep.release();
-    ix.deep_depth = 0;
     lut_literal_kernel<IdxT><<<unsigned(ceil_div(kLutSize, 128)), 128, 0, s>>>(ctx->d_text.p, ctx->n1, ix.sa.p, m1, ix.lut_lo.p, ix.lut_hi.p);
     KERNEL_CHECK();
     count_launch();
@@ -499,9 +528,19 @@ void upload_from_i64(const i64* h, T* d, u64 n, cudaStream_t s) {
     }
 }
 
+// the divsufsort64 drop-in: suffix array of T[0, n) built on the device with IdxT entries
 template <typename IdxT>
-i64 check_sa_t(asgart_b200_ctx* ctx) {
-    auto& ix = IxOf<IdxT>::get(ctx);
+void divsufsort_t(const u8* T, i64* SA, u64 n, cudaStream_t s) {
+    DevBuf<u8> d_text(n, s);
+    CUDA_CHECK(cudaMemcpyAsync(d_text.p, T, n, cudaMemcpyHostToDevice, s));
+    DevBuf<IdxT> sa(n, s), rank(n, s);
+    build_suffix_array<IdxT>(d_text.p, n, sa.p, rank.p, s, nullptr);
+    rank.release();
+    download_as_i64(sa.p, SA, n, s);
+}
+
+template <typename IdxT>
+i64 check_sa_t(asgart_b200_ctx* ctx, const Index<IdxT>& ix) {
     const u64 n1 = ctx->n1;
     cudaStream_t s = ctx->stream;
     DevBuf<IdxT> isa(n1, s);
@@ -549,8 +588,7 @@ __global__ void __launch_bounds__(256) sa_fingerprint_kernel(const IdxT* __restr
     if ((threadIdx.x & 31u) == 0) atomicAdd(out, (unsigned long long)acc);
 }
 template <typename IdxT>
-u64 sa_fingerprint_t(asgart_b200_ctx* ctx) {
-    auto& ix = IxOf<IdxT>::get(ctx);
+u64 sa_fingerprint_t(asgart_b200_ctx* ctx, const Index<IdxT>& ix) {
     cudaStream_t s = ctx->stream;
     DevBuf<unsigned long long> acc(1, s);
     acc.zero();
@@ -613,8 +651,7 @@ void ensure_needle(asgart_b200_ctx* ctx, int mode) {
 // the probes it left to the literal search. Reads the counters back (one sync). mode: the needle image (PackMode).
 // Returns the number of probes answered from the sorted keys.
 template <typename IdxT>
-u64 run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, int mode, unsigned long long* h_ctr) {
-    auto& ix = IxOf<IdxT>::get(ctx);
+u64 run_probe_kernels(asgart_b200_ctx* ctx, const Index<IdxT>& ix, ProbeParams<IdxT>& P, int mode, unsigned long long* h_ctr) {
     cudaStream_t s = ctx->stream;
     const u64 np = P.p_end - P.p_begin;
     DevBuf<u32> q6(ceil_div(kLutSize, 32), s);
@@ -667,8 +704,7 @@ u64 run_probe_kernels(asgart_b200_ctx* ctx, ProbeParams<IdxT>& P, int mode, unsi
 
 // the ProbeParams fields of every probe search over [p_begin, p_end) of the plan: text and needle images, index, chunks
 template <typename IdxT>
-ProbeParams<IdxT> probe_params(asgart_b200_ctx* ctx, const ChunkPlan& plan, u64 p_begin, u64 p_end) {
-    auto& ix = IxOf<IdxT>::get(ctx);
+ProbeParams<IdxT> probe_params(asgart_b200_ctx* ctx, const Index<IdxT>& ix, const ChunkPlan& plan, u64 p_begin, u64 p_end) {
     ProbeParams<IdxT> P{};
     P.PT = ctx->d_pt.p;
     P.PN = plan.mode == PACK_DIRECT ? ctx->d_pt.p : ctx->d_pn.p;
@@ -680,9 +716,9 @@ ProbeParams<IdxT> probe_params(asgart_b200_ctx* ctx, const ChunkPlan& plan, u64 
 }
 
 template <typename IdxT>
-void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_settings* st, u64 p_begin, u64 p_end, StageA& A) {
+void run_stage_a(asgart_b200_ctx* ctx, const Index<IdxT>& ix, const ChunkPlan& plan, const asgart_b200_settings* st, u64 p_begin, u64 p_end,
+                 StageA& A) {
     NvtxRange nv("search/stage A: probe search + emit");
-    auto& ix = IxOf<IdxT>::get(ctx);
     cudaStream_t s = ctx->stream;
     A.p_begin = p_begin; A.p_end = p_end;
     const u64 np = p_end - p_begin;
@@ -693,13 +729,13 @@ void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
     DevBuf<u32> out_surv(np, s);
     DevBuf<unsigned long long> counters(CTR_COUNT, s);
     counters.zero();
-    ProbeParams<IdxT> P = probe_params<IdxT>(ctx, plan, p_begin, p_end);
+    ProbeParams<IdxT> P = probe_params(ctx, ix, plan, p_begin, p_end);
     P.reverse = st->reverse ? 1 : 0; P.max_card = st->max_cardinality;
     P.out_lo = out_lo.p; P.out_raw = out_raw.p; P.out_surv = out_surv.p; P.proc_bits = A.bits.p; P.counters = counters.p;
     unsigned long long h_ctr[CTR_COUNT];
-    ctx->t_probe.begin();
-    const u64 n_keys = run_probe_kernels<IdxT>(ctx, P, plan.mode, h_ctr);
-    ctx->t_probe.end(1, h_ctr[CTR_ALG_BYTES]);
+    ctx->fam[FAM_PROBE].begin();
+    const u64 n_keys = run_probe_kernels(ctx, ix, P, plan.mode, h_ctr);
+    ctx->fam[FAM_PROBE].end(1, h_ctr[CTR_ALG_BYTES]);
     ctx->st.n_probes += np;
     ctx->st.n_searched += h_ctr[CTR_SEARCHED];
     ctx->st.n_skipped_n += h_ctr[CTR_SKIP_N];
@@ -708,7 +744,7 @@ void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
     ctx->n_probe_keys += n_keys;
 
     // match offsets + event list + emission, fused into one scan
-    ctx->t_emit.begin();
+    ctx->fam[FAM_EMIT].begin();
     const u32* surv = out_surv.p;
     auto in = [surv] __device__(u64 o) { const u32 v = surv[o]; return Sum2(u64(v), v ? 1ull : 0ull); };
     DevBuf<Sum2> d_total(1, s);
@@ -739,7 +775,7 @@ void run_stage_a(asgart_b200_ctx* ctx, const ChunkPlan& plan, const asgart_b200_
             count_launch();
         }
     }
-    ctx->t_emit.end(3, 0);
+    ctx->fam[FAM_EMIT].end(3, 0);
 }
 
 // ---------------------------------------------------------------------------------------------- post-steps
@@ -960,8 +996,7 @@ int search_stage_a(asgart_b200_ctx* ctx, const asgart_b200_chunk* chunks, i64 n_
     shard_range(plan.total_probes, shard, n_shards, b, e);
     EventTimer ts(ctx->stream);
     ts.start();
-    if (ctx->idx_bits == 32) run_stage_a<u32>(ctx, plan, st, b, e, A);
-    else run_stage_a<u64>(ctx, plan, st, b, e, A);
+    with_index(ctx, [&](auto& ix) { run_stage_a(ctx, ix, plan, st, b, e, A); });
     in_timer();
     ts.stop();
     ctx->st.ms_search += ts.ms();
@@ -1056,25 +1091,24 @@ int32_t enable_peer_access(const asgart_b200_ctx* const* ctxs, int n, asgart_b20
 }
 
 void fold_family_timers(asgart_b200_ctx* ctx) {
-    ctx->t_sort.drain(); ctx->t_gather.drain(); ctx->t_rank.drain(); ctx->t_probe.drain(); ctx->t_emit.drain(); ctx->t_scatter.drain(); ctx->t_scatter_main.drain();
-    ctx->t_msd0.drain(); ctx->t_msd_hist.drain(); ctx->t_msd_local.drain();
+    for (FamilyTimer& t : ctx->fam) t.drain();
+    const FamilyTimer* f = ctx->fam;
     asgart_b200_stats& S = ctx->st;
-    S.ms_msd_scatter0 = ctx->t_msd0.total_ms; S.bytes_msd_scatter0 = ctx->t_msd0.bytes;
-    S.ms_msd_hist = ctx->t_msd_hist.total_ms; S.bytes_msd_hist = ctx->t_msd_hist.bytes;
-    S.ms_msd_local = ctx->t_msd_local.total_ms; S.bytes_msd_local = ctx->t_msd_local.bytes; S.launches_msd_local = ctx->t_msd_local.launches;
-    S.ms_sa_sort = ctx->t_sort.total_ms; S.launches_sa_sort = ctx->t_sort.launches; S.bytes_sa_sort = ctx->t_sort.bytes;
-    S.ms_sa_gather = ctx->t_gather.total_ms; S.launches_sa_gather = ctx->t_gather.launches; S.bytes_sa_gather = ctx->t_gather.bytes;
-    S.ms_sa_rank = ctx->t_rank.total_ms;
-    S.ms_probe = ctx->t_probe.total_ms; S.launches_probe = ctx->t_probe.launches; S.bytes_probe = ctx->t_probe.bytes;
-    S.ms_emit = ctx->t_emit.total_ms;
-    S.ms_sa_scatter_main = ctx->t_scatter_main.total_ms; S.launches_sa_scatter_main = ctx->t_scatter_main.launches;
-    S.bytes_sa_scatter_main = ctx->t_scatter_main.bytes;
-    S.ms_sa_scatter = ctx->t_scatter.total_ms + S.ms_sa_scatter_main; S.launches_sa_scatter = ctx->t_scatter.launches + S.launches_sa_scatter_main;
-    S.bytes_sa_scatter = ctx->t_scatter.bytes + S.bytes_sa_scatter_main;
-    ctx->t_locate.drain();
-    S.ms_locate = ctx->t_locate.total_ms;
+    S.ms_msd_scatter0 = f[FAM_MSD0].total_ms; S.bytes_msd_scatter0 = f[FAM_MSD0].bytes;
+    S.ms_msd_hist = f[FAM_MSD_HIST].total_ms; S.bytes_msd_hist = f[FAM_MSD_HIST].bytes;
+    S.ms_msd_local = f[FAM_MSD_LOCAL].total_ms; S.bytes_msd_local = f[FAM_MSD_LOCAL].bytes; S.launches_msd_local = f[FAM_MSD_LOCAL].launches;
+    S.ms_sa_sort = f[FAM_SORT].total_ms; S.launches_sa_sort = f[FAM_SORT].launches; S.bytes_sa_sort = f[FAM_SORT].bytes;
+    S.ms_sa_gather = f[FAM_GATHER].total_ms; S.launches_sa_gather = f[FAM_GATHER].launches; S.bytes_sa_gather = f[FAM_GATHER].bytes;
+    S.ms_sa_rank = f[FAM_RANK].total_ms;
+    S.ms_probe = f[FAM_PROBE].total_ms; S.launches_probe = f[FAM_PROBE].launches; S.bytes_probe = f[FAM_PROBE].bytes;
+    S.ms_emit = f[FAM_EMIT].total_ms;
+    S.ms_sa_scatter_main = f[FAM_SCATTER_MAIN].total_ms; S.launches_sa_scatter_main = f[FAM_SCATTER_MAIN].launches;
+    S.bytes_sa_scatter_main = f[FAM_SCATTER_MAIN].bytes;
+    S.ms_sa_scatter = f[FAM_SCATTER].total_ms + S.ms_sa_scatter_main; S.launches_sa_scatter = f[FAM_SCATTER].launches + S.launches_sa_scatter_main;
+    S.bytes_sa_scatter = f[FAM_SCATTER].bytes + S.bytes_sa_scatter_main;
+    S.ms_locate = f[FAM_LOCATE].total_ms;
     S.launches_total = ctx->launches.total;
-    S.sa_index_bits = u64(ctx->idx_bits);
+    S.sa_index_bits = std::holds_alternative<Index<u32>>(ctx->ix) ? 32 : std::holds_alternative<Index<u64>>(ctx->ix) ? 64 : 0;
 }
 
 
@@ -1105,8 +1139,8 @@ void loc_copy(asgart_b200_ctx* ctx, void* dst, const void* src, size_t bytes, bo
 
 // returns false when the positions do not fit in host memory
 template <typename IdxT>
-bool locate_t(asgart_b200_ctx* ctx, const u8* patterns, const u64* offsets, u64 n, i64 max_hits, asgart_b200_hits& H) {
-    auto& ix = IxOf<IdxT>::get(ctx);
+bool locate_t(asgart_b200_ctx* ctx, const Index<IdxT>& ix, const u8* patterns, const u64* offsets, u64 n, i64 max_hits,
+              asgart_b200_hits& H) {
     cudaStream_t s = ctx->stream;
     const bool literal = ctx->sa_len != ctx->n1;   // --trim: the literal search (SURVEY Q9)
     const u64 cap = max_hits < 0 ? ~u64(0) : u64(max_hits);
@@ -1143,7 +1177,7 @@ bool locate_t(asgart_b200_ctx* ctx, const u8* patterns, const u64* offsets, u64 
         P.lut_lo = ix.lut_lo.p; P.lut_hi = ix.lut_hi.p; P.deep = ix.deep.p; P.deep_depth = ix.deep.p ? ix.deep_depth : 0;
         P.pat = d_pat.p; P.PP = d_pp.p; P.off = d_off.p; P.cut = d_cut.p;
         P.first = d_first.p; P.count = d_count.p; P.alg_bytes = d_alg.p;
-        ctx->t_locate.begin();
+        ctx->fam[FAM_LOCATE].begin();
         u64 launches = 0;
         if (literal) {
             P.list = nullptr; P.n_list = np;
@@ -1164,7 +1198,7 @@ bool locate_t(asgart_b200_ctx* ctx, const u8* patterns, const u64* offsets, u64 
                 ++launches;
             }
         }
-        ctx->t_locate.end(launches, 0);
+        ctx->fam[FAM_LOCATE].end(launches, 0);
         count_launch(launches);
         loc_copy(ctx, H.first.data() + p0, d_first.p, np * 8, false);
         loc_copy(ctx, H.count.data() + p0, d_count.p, np * 8, false);
@@ -1187,11 +1221,11 @@ bool locate_t(asgart_b200_ctx* ctx, const u8* patterns, const u64* offsets, u64 
             DevBuf<i64> d_out(std::min(hs, kLocWindow), s);
             for (u64 w0 = 0; w0 < hs; w0 += kLocWindow) {
                 const u64 w1 = std::min(hs, w0 + kLocWindow);
-                ctx->t_locate.begin();
+                ctx->fam[FAM_LOCATE].begin();
                 locate_copy_kernel<IdxT><<<unsigned(ceil_div(np * 32, 256)), 256, 0, s>>>(ix.sa.p, d_first.p, d_count.p, d_moff.p, np,
                                                                                          cap, w0, w1, d_out.p);
                 KERNEL_CHECK();
-                ctx->t_locate.end(1, 0);
+                ctx->fam[FAM_LOCATE].end(1, 0);
                 count_launch();
                 loc_copy(ctx, H.positions.data() + hits + w0, d_out.p, (w1 - w0) * 8, false);
             }
@@ -1238,10 +1272,7 @@ int32_t asgart_b200_ctx_create(int32_t device, asgart_b200_ctx** out) {
         CUDA_CHECK(cudaDeviceGetDefaultMemPool(&pool, device));
         u64 thr = ~u64(0);
         CUDA_CHECK(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr));
-        ctx->t_sort.init(ctx->stream); ctx->t_gather.init(ctx->stream); ctx->t_rank.init(ctx->stream);
-        ctx->t_probe.init(ctx->stream); ctx->t_emit.init(ctx->stream); ctx->t_scatter.init(ctx->stream); ctx->t_scatter_main.init(ctx->stream);
-        ctx->t_msd0.init(ctx->stream); ctx->t_msd_hist.init(ctx->stream); ctx->t_msd_local.init(ctx->stream);
-        ctx->t_locate.init(ctx->stream);
+        for (FamilyTimer& t : ctx->fam) t.init(ctx->stream);
         CUDA_CHECK(cudaEventCreate(&ctx->ev_a)); CUDA_CHECK(cudaEventCreate(&ctx->ev_b));
     } catch (const CudaError& e) {
         int code = e.code;
@@ -1260,8 +1291,7 @@ void asgart_b200_ctx_destroy(asgart_b200_ctx* ctx) {
                 (unsigned long long)g_host_stalls.allocs, g_host_stalls.alloc_ms, (unsigned long long)g_host_stalls.syncs, g_host_stalls.sync_ms);
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
-    ctx->t_sort.destroy(); ctx->t_gather.destroy(); ctx->t_rank.destroy(); ctx->t_probe.destroy(); ctx->t_emit.destroy(); ctx->t_scatter.destroy(); ctx->t_scatter_main.destroy();
-    ctx->t_msd0.destroy(); ctx->t_msd_hist.destroy(); ctx->t_msd_local.destroy(); ctx->t_locate.destroy();
+    for (FamilyTimer& t : ctx->fam) t.destroy();
     if (ctx->loc_stage) cudaFreeHost(ctx->loc_stage);
     if (ctx->ev_a) cudaEventDestroy(ctx->ev_a);
     if (ctx->ev_b) cudaEventDestroy(ctx->ev_b);
@@ -1275,8 +1305,7 @@ void asgart_b200_ctx_destroy(asgart_b200_ctx* ctx) {
         if (ctx->stage_ev[i]) cudaEventDestroy(ctx->stage_ev[i]);
     }
     ctx->d_text.release(); ctx->d_pt.release(); ctx->d_pn.release(); ctx->shard_blob.release();
-    ctx->ix32 = Index32();
-    ctx->ix64 = Index64();
+    ctx->ix = std::monostate();
     cudaStreamSynchronize(ctx->stream);
     cudaStreamDestroy(ctx->stream);
     delete ctx;
@@ -1294,9 +1323,7 @@ int32_t asgart_b200_ctx_set_index_bits(asgart_b200_ctx* ctx, int32_t bits) {
 int32_t asgart_b200_ctx_load_strand(asgart_b200_ctx* ctx, const uint8_t* T, int64_t n_plus_1) {
     return guarded(ctx, [&]() -> int32_t {
         if (!T || n_plus_1 < 1) return fail(ctx, ASGART_B200_EINVAL, "null strand or n_plus_1 < 1");
-        ctx->have_strand = ctx->have_index = false;
-        drop_sorted_keys(ctx);
-        ctx->pn_mode = -1;
+        forget_strand(ctx);
         ctx->n1 = u64(n_plus_1);
         EventTimer th(ctx->stream);
         th.start();
@@ -1327,9 +1354,7 @@ int32_t asgart_b200_ctx_load_strand(asgart_b200_ctx* ctx, const uint8_t* T, int6
 // ---- GPU-side FASTA ingest (fasta_ingest.cuh) -----------------------------------------------------------------
 int32_t asgart_b200_ctx_ingest_begin(asgart_b200_ctx* ctx) {
     return guarded(ctx, [&]() -> int32_t {
-        ctx->have_strand = ctx->have_index = false;
-        drop_sorted_keys(ctx);
-        ctx->pn_mode = -1;
+        forget_strand(ctx);
         ctx->pieces.clear();
         ctx->ingesting = true;
         return ASGART_B200_OK;
@@ -1489,9 +1514,7 @@ int32_t asgart_b200_ctx_copy_strand(asgart_b200_ctx* dst, const asgart_b200_ctx*
         const int32_t prc = enable_peer_access(pair, 2, dst);
         if (prc) return prc;
         CUDA_CHECK(cudaSetDevice(dst->device));
-        dst->have_strand = dst->have_index = false;
-        drop_sorted_keys(dst);
-        dst->pn_mode = -1;
+        forget_strand(dst);
         dst->n1 = src->n1;
         // src's strand is complete: its load or ingest synchronised its stream before it set have_strand
         dst->d_text.alloc(dst->n1, dst->stream);
@@ -1503,15 +1526,7 @@ int32_t asgart_b200_ctx_copy_strand(asgart_b200_ctx* dst, const asgart_b200_ctx*
 int32_t asgart_b200_ctx_build_index(asgart_b200_ctx* ctx) {
     return guarded(ctx, [&]() -> int32_t {
         if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "build_index before load_strand");
-        ctx->have_index = false;
-        ctx->idx_bits = pick_bits(ctx);
-        if (ctx->idx_bits == 32 && ctx->n1 >= 0xFFFFFFFEull) return fail(ctx, ASGART_B200_EINVAL, "32-bit indices need n+1 < 2^32-2");
-        if (ctx->idx_bits == 32) { ctx->ix64 = Index64(); build_index_t<u32>(ctx); }
-        else { ctx->ix32 = Index32(); build_index_t<u64>(ctx); }
-        CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-        ctx->sa_len = ctx->n1;
-        ctx->have_index = true;
-        return ASGART_B200_OK;
+        return install_index(ctx, ctx->n1, [&](auto& ix) { build_index_t(ctx, ix); });
     });
 }
 
@@ -1522,15 +1537,7 @@ int32_t asgart_b200_ctx_build_index_trim(asgart_b200_ctx* ctx, uint64_t a, uint6
         if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "build_index_trim before load_strand");
         if (ctx->group && ctx->group->world > 1) return fail(ctx, ASGART_B200_ESTATE, "--trim builds on one device");
         if (!(a < b) || b > ctx->n1 - 1) return fail(ctx, ASGART_B200_EINVAL, "trim needs start < stop <= strand length (see asgart_b200_effective_trim)");
-        ctx->have_index = false;
-        ctx->idx_bits = pick_bits(ctx);
-        if (ctx->idx_bits == 32 && ctx->n1 >= 0xFFFFFFFEull) return fail(ctx, ASGART_B200_EINVAL, "32-bit indices need n+1 < 2^32-2");
-        if (ctx->idx_bits == 32) { ctx->ix64 = Index64(); build_index_trim_t<u32>(ctx, a, b); }
-        else { ctx->ix32 = Index32(); build_index_trim_t<u64>(ctx, a, b); }
-        CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-        ctx->sa_len = b - a + 1;
-        ctx->have_index = true;
-        return ASGART_B200_OK;
+        return install_index(ctx, b - a + 1, [&](auto& ix) { build_index_trim_t(ctx, ix, a, b); });
     });
 }
 
@@ -1660,23 +1667,11 @@ int32_t asgart_b200_ctx_upload_sa(asgart_b200_ctx* ctx, const int64_t* SA) {
     return guarded(ctx, [&]() -> int32_t {
         if (!ctx->have_strand) return fail(ctx, ASGART_B200_ESTATE, "upload_sa before load_strand");
         if (!SA) return fail(ctx, ASGART_B200_EINVAL, "null SA");
-        ctx->have_index = false;
-        ctx->idx_bits = pick_bits(ctx);
-        if (ctx->idx_bits == 32) {
-            ctx->ix64 = Index64();
-            ctx->ix32.sa.alloc(ctx->n1, ctx->stream);
-            upload_from_i64<u32>(SA, ctx->ix32.sa.p, ctx->n1, ctx->stream);
-            build_lut<u32>(ctx);
-        } else {
-            ctx->ix32 = Index32();
-            ctx->ix64.sa.alloc(ctx->n1, ctx->stream);
-            upload_from_i64<u64>(SA, ctx->ix64.sa.p, ctx->n1, ctx->stream);
-            build_lut<u64>(ctx);
-        }
-        CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-        ctx->sa_len = ctx->n1;
-        ctx->have_index = true;
-        return ASGART_B200_OK;
+        return install_index(ctx, ctx->n1, [&](auto& ix) {
+            ix.sa.alloc(ctx->n1, ctx->stream);
+            upload_from_i64(SA, ix.sa.p, ctx->n1, ctx->stream);
+            build_lut(ctx, ix);
+        });
     });
 }
 
@@ -1684,8 +1679,7 @@ int32_t asgart_b200_ctx_download_sa(asgart_b200_ctx* ctx, int64_t* SA) {
     return guarded(ctx, [&]() -> int32_t {
         if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "download_sa before build_index");
         if (!SA) return fail(ctx, ASGART_B200_EINVAL, "null SA");
-        if (ctx->idx_bits == 32) download_as_i64<u32>(ctx->ix32.sa.p, SA, ctx->sa_len, ctx->stream);
-        else download_as_i64<u64>(ctx->ix64.sa.p, SA, ctx->sa_len, ctx->stream);
+        with_index(ctx, [&](auto& ix) { download_as_i64(ix.sa.p, SA, ctx->sa_len, ctx->stream); });
         return ASGART_B200_OK;
     });
 }
@@ -1695,7 +1689,7 @@ int32_t asgart_b200_ctx_check_sa(asgart_b200_ctx* ctx, int64_t* n_bad) {
         if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "check_sa before build_index");
         if (!n_bad) return fail(ctx, ASGART_B200_EINVAL, "null output");
         if (ctx->sa_len != ctx->n1) return fail(ctx, ASGART_B200_ESTATE, "check_sa: the index was built with --trim (it is not a suffix array of the strand)");
-        if (ctx->idx_bits == 32) *n_bad = check_sa_t<u32>(ctx); else *n_bad = check_sa_t<u64>(ctx);
+        *n_bad = with_index(ctx, [&](auto& ix) { return check_sa_t(ctx, ix); });
         return ASGART_B200_OK;
     });
 }
@@ -1704,7 +1698,7 @@ int32_t asgart_b200_ctx_sa_fingerprint(asgart_b200_ctx* ctx, uint64_t* fingerpri
     return guarded(ctx, [&]() -> int32_t {
         if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "sa_fingerprint before build_index");
         if (!fingerprint) return fail(ctx, ASGART_B200_EINVAL, "null output");
-        *fingerprint = ctx->idx_bits == 32 ? sa_fingerprint_t<u32>(ctx) : sa_fingerprint_t<u64>(ctx);
+        *fingerprint = with_index(ctx, [&](auto& ix) { return sa_fingerprint_t(ctx, ix); });
         return ASGART_B200_OK;
     });
 }
@@ -1713,13 +1707,10 @@ int32_t asgart_b200_ctx_download_lut(asgart_b200_ctx* ctx, int64_t* lo, int64_t*
     return guarded(ctx, [&]() -> int32_t {
         if (!ctx->have_index) return fail(ctx, ASGART_B200_ESTATE, "download_lut before build_index");
         if (!lo || !hi) return fail(ctx, ASGART_B200_EINVAL, "null output");
-        if (ctx->idx_bits == 32) {
-            download_as_i64<u32>(ctx->ix32.lut_lo.p, lo, kLutSize, ctx->stream);
-            download_as_i64<u32>(ctx->ix32.lut_hi.p, hi, kLutSize, ctx->stream);
-        } else {
-            download_as_i64<u64>(ctx->ix64.lut_lo.p, lo, kLutSize, ctx->stream);
-            download_as_i64<u64>(ctx->ix64.lut_hi.p, hi, kLutSize, ctx->stream);
-        }
+        with_index(ctx, [&](auto& ix) {
+            download_as_i64(ix.lut_lo.p, lo, kLutSize, ctx->stream);
+            download_as_i64(ix.lut_hi.p, hi, kLutSize, ctx->stream);
+        });
         return ASGART_B200_OK;
     });
 }
@@ -1738,17 +1729,15 @@ int32_t asgart_b200_ctx_probe_ranges(asgart_b200_ctx* ctx, const asgart_b200_chu
         if (n_probes == 0) return ASGART_B200_OK;
         ensure_needle(ctx, plan.mode);
         DevBuf<i64> d_lo(n_probes, ctx->stream), d_hi(n_probes, ctx->stream);
-        auto launch = [&](auto tag) {
-            using IdxT = decltype(tag);
-            ProbeParams<IdxT> P = probe_params<IdxT>(ctx, plan, 0, u64(n_probes));
+        with_index(ctx, [&](auto& ix) {
+            auto P = probe_params(ctx, ix, plan, 0, u64(n_probes));
             P.rng_lo = d_lo.p; P.rng_hi = d_hi.p;
             DevBuf<unsigned long long> counters(CTR_COUNT, ctx->stream);
             counters.zero();
             P.counters = counters.p;
             unsigned long long h_ctr[CTR_COUNT];
-            ctx->n_probe_keys += run_probe_kernels<IdxT>(ctx, P, plan.mode, h_ctr);
-        };
-        if (ctx->idx_bits == 32) launch(u32(0)); else launch(u64(0));
+            ctx->n_probe_keys += run_probe_kernels(ctx, ix, P, plan.mode, h_ctr);
+        });
         CUDA_CHECK(cudaMemcpyAsync(lo, d_lo.p, n_probes * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_CHECK(cudaMemcpyAsync(hi, d_hi.p, n_probes * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
@@ -1922,8 +1911,7 @@ int32_t asgart_b200_ctx_locate(asgart_b200_ctx* ctx, const uint8_t* patterns, co
             if (offsets[i + 1] < offsets[i]) return fail(ctx, ASGART_B200_EINVAL, "locate: offsets are not non-decreasing");
         if (n > 0 && offsets[n] > offsets[0] && !patterns) return fail(ctx, ASGART_B200_EINVAL, "locate: null patterns");
         std::unique_ptr<asgart_b200_hits> H(new asgart_b200_hits());
-        const bool ok = ctx->idx_bits == 32 ? locate_t<u32>(ctx, patterns, offsets, n, max_hits, *H)
-                                            : locate_t<u64>(ctx, patterns, offsets, n, max_hits, *H);
+        const bool ok = with_index(ctx, [&](auto& ix) { return locate_t(ctx, ix, patterns, offsets, n, max_hits, *H); });
         if (!ok) return fail(ctx, ASGART_B200_ENOMEM, "locate: the reported positions do not fit in host memory (lower max_hits)");
         *out = H.release();
         return ASGART_B200_OK;
@@ -1954,8 +1942,7 @@ void asgart_b200_ctx_reset_stats(asgart_b200_ctx* ctx) {
     if (!ctx) return;
     try {
         cudaSetDevice(ctx->device);
-        ctx->t_sort.reset(); ctx->t_gather.reset(); ctx->t_rank.reset(); ctx->t_probe.reset(); ctx->t_emit.reset(); ctx->t_scatter.reset(); ctx->t_scatter_main.reset();
-        ctx->t_msd0.reset(); ctx->t_msd_hist.reset(); ctx->t_msd_local.reset(); ctx->t_locate.reset();
+        for (FamilyTimer& t : ctx->fam) t.reset();
     } catch (...) {}
     ctx->launches.total = 0;
     ctx->st = asgart_b200_stats{};
@@ -1989,23 +1976,10 @@ int32_t asgart_b200_divsufsort64_ex(const uint8_t* T, int64_t* SA, int64_t n, in
     try {
         CUDA_CHECK(cudaSetDevice(device));
         CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-        int bits = index_bits ? index_bits : (u64(n) < 0xFFFFFFFEull ? 32 : 64);
-        {
-            DevBuf<u8> d_text(u64(n), s);
-            CUDA_CHECK(cudaMemcpyAsync(d_text.p, T, size_t(n), cudaMemcpyHostToDevice, s));
-            if (bits == 32) {
-                if (u64(n) >= 0xFFFFFFFEull) { cudaStreamDestroy(s); return ASGART_B200_EINVAL; }
-                DevBuf<u32> sa(u64(n), s), rank(u64(n), s);
-                build_suffix_array<u32>(d_text.p, u64(n), sa.p, rank.p, s, nullptr);
-                rank.release();
-                download_as_i64<u32>(sa.p, SA, u64(n), s);
-            } else {
-                DevBuf<u64> sa(u64(n), s), rank(u64(n), s);
-                build_suffix_array<u64>(d_text.p, u64(n), sa.p, rank.p, s, nullptr);
-                rank.release();
-                download_as_i64<u64>(sa.p, SA, u64(n), s);
-            }
-        }
+        const int bits = index_bits ? index_bits : (fits_u32_index(u64(n)) ? 32 : 64);   // any width but 32 builds with 64 bits
+        if (bits == 32 && !fits_u32_index(u64(n))) { cudaStreamDestroy(s); return ASGART_B200_EINVAL; }
+        if (bits == 32) divsufsort_t<u32>(T, SA, u64(n), s);
+        else divsufsort_t<u64>(T, SA, u64(n), s);
         CUDA_CHECK(cudaStreamSynchronize(s));
         cudaStreamDestroy(s);
         return ASGART_B200_OK;
